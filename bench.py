@@ -48,7 +48,29 @@ def parse():
     ap.add_argument("--tiles", default="static", choices=["static", "dynamic"],
                     help="N > 1: static interleaved tile groups, or dynamic stealing of super-tile ranges from the shared-memory work counter")
     ap.add_argument("--ref-spp", type=int, default=8, help="--impl reference: samples per pixel per step (bounded sample of the GPU arm's step)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the film of the last timed step to DIR/*.npy (float32; a seeded pixel sample when the film exceeds 64 MB)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_MAX_PIXELS = 1 << 21  # 32 MB of float32 RGBW (+ 16 MB of float64 pixel indices when sampled): under 64 MB in all
+
+
+def dump_outputs(out_dir, rgbw, width, height):
+    """The film accumulator (per pixel: filter-weighted R, G, B and the filter weight sum) that the render call handed back for the last
+    timed step.  Films above DUMP_MAX_PIXELS are written as a fixed, seeded sample of pixels, with their row-major indices."""
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    rgbw = np.asarray(rgbw, np.float32).reshape(height * width, 4)
+    if len(rgbw) <= DUMP_MAX_PIXELS:
+        np.save(out / "film_rgbw.npy", rgbw.reshape(height, width, 4))
+        return
+    idx = np.sort(np.random.default_rng(0).choice(len(rgbw), DUMP_MAX_PIXELS, replace=False))
+    np.save(out / "film_rgbw_sample.npy", rgbw[idx])
+    np.save(out / "film_pixel_index.npy", idx.astype(np.float64))
 
 
 def make_setup(pkg, name):
@@ -191,9 +213,11 @@ def main():
         samples = 0
         for k in range(args.steps):
             b = (args.warmup + k) * ref_spp
-            _, st = O.render(setup.flat, integ, nthreads=nth, sample_range=(b, b + ref_spp))
+            rgbw, st = O.render(setup.flat, integ, nthreads=nth, sample_range=(b, b + ref_spp))
             samples += st["camera_rays"]
         dt = time.time() - t0
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, rgbw, film.width, film.height)
         v = samples / dt
         print(json.dumps({"impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
                           "ms_per_step": dt / args.steps * 1e3, "higher_is_better": True, "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -285,6 +309,8 @@ def main():
     sync()
     ms = e0.elapsed_time(e1)
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:  # film_t holds the last timed step (summed over ranks); the e2e leg below reuses it
+        dump_outputs(args.dump_outputs, film_t.cpu().numpy(), film.width, film.height)
     vals = torch.tensor([ms, tot["camera"], tot["closest"], tot["shadow"], tot["launches"]], dtype=torch.float64, device="cuda")
     if world > 1:
         mx = vals.clone(); dist.all_reduce(mx, op=dist.ReduceOp.MAX)

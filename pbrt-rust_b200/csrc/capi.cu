@@ -713,9 +713,6 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
     DevScene& ds = sc->dev;
     ds.n_slots = (uint32_t)np;
     ds.n_lights = (uint32_t)d->n_lights;
-    ds.n_sphere_lights = 0;
-    for (uint64_t i = 0; i < d->n_lights; ++i)
-        if (d->lights[i].type == PBRT_B200_LIGHT_DIFFUSE && d->lights[i].shape_kind == PBRT_B200_SHAPE_SPHERE) ds.n_sphere_lights += 1;
     ds.n_materials = (uint32_t)d->n_materials;
     if (nn) {
         std::memcpy(ds.root_box, d->nodes[0].bounds, sizeof ds.root_box);
@@ -779,6 +776,10 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
     lap("h2d staged");
     if ((rc = join_checks())) { pbrt_b200_scene_destroy(sc); return rc; }
     lap("checks joined");
+    // read on this thread only now: until the table checks have passed, `lights` may be null with a non-zero count
+    ds.n_sphere_lights = 0;
+    for (uint64_t i = 0; i < d->n_lights; ++i)
+        if (d->lights[i].type == PBRT_B200_LIGHT_DIFFUSE && d->lights[i].shape_kind == PBRT_B200_SHAPE_SPHERE) ds.n_sphere_lights += 1;
     ds.root_ref = root_ref;
     ds.n_fat = n_interior;
     if (np && err == cudaSuccess)

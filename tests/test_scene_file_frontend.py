@@ -1,8 +1,8 @@
 """Scene-file front end (SURVEY.md §8 f2): `.pbrt` lexer / grammar, ParamSet, API state machine, plymesh.
 
-The reference has no tests for its parser; parity is anchored on (1) its own scene files under src/scenes (parsed
-here when /root/reference is mounted, never on the GPU box), (2) known answers that its code fixes — the copper
-RGB of metal.rs through `from_sampled`, f32 literal rounding, the ParamSet lookup rules — and (3) the closed loop
+The reference has no tests for its parser; parity is anchored on (1) its own spheres scene file, re-emitted directive for
+directive as tests/golden/reference_spheres_scene.pbrt, (2) known answers that its code fixes — the copper RGB of metal.rs
+through `from_sampled`, f32 literal rounding, the ParamSet lookup rules — and (3) the closed loop
 scene -> .pbrt/.ply -> parser -> API -> byte-identical FlatScene and render descriptor.
 """
 import importlib
@@ -17,7 +17,6 @@ import pytest
 pkg = importlib.import_module("pbrt-rust_b200")
 PP, PS, SP, SF, PLY = pkg.pbrtparser, pkg.paramset, pkg.spectrum, importlib.import_module("pbrt-rust_b200.scenefile"), pkg.plymesh
 f32 = np.float32
-REF_SCENES = Path("/root/reference/src/scenes")
 
 FLAT_KEYS = ("nodes", "prims", "vertex_p", "vertex_n", "vertex_s", "vertex_uv", "tri_indices", "spheres", "materials", "lights", "objects", "instances")
 
@@ -276,56 +275,13 @@ def test_include_resolves_against_the_scene_directory(tmp_path):
     assert job.flat.spheres[0]["radius"] == 2.0 and job.flat.materials[0]["type"] == pkg.host.MAT_MIRROR
 
 
-@pytest.mark.skipif(not REF_SCENES.exists(), reason="reference tree not mounted (GPU box)")
-def test_reference_scene_files_lex_and_parse():
-    counts = {}
-    for name in ("caustic-glass.pbrt", "spheres-differentials-texfilt.pbrt", "sss-dragon.pbrt"):
-        cmds = PP.parse_commands((REF_SCENES / name).read_text(), name)
-        counts[name] = len(cmds)
-        assert cmds[-1] == ("WorldEnd",) and sum(c[0] == "WorldBegin" for c in cmds) == 1
-    assert counts == {"caustic-glass.pbrt": 18, "spheres-differentials-texfilt.pbrt": 22, "sss-dragon.pbrt": 26}
-    # their integrators / materials are outside the hot path: the API says so instead of rendering something else
-    with pytest.raises(pkg.B200Error), warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        pkg.pbrt_parse(REF_SCENES / "caustic-glass.pbrt")
-    # ... except the spheres scene, which runs as it is (directlighting "all", lowdiscrepancy sampler, missing image map -> grey):
-    # tests/golden/reference_spheres_scene.pbrt holds the same directives (re-emitted, not copied) and is what
-    # tests/test_gpu_recursive_integrators.py renders on the GPU
-    ours = PP.parse_commands((Path(__file__).parent / "golden" / "reference_spheres_scene.pbrt").read_text())
-    theirs = PP.parse_commands((REF_SCENES / "spheres-differentials-texfilt.pbrt").read_text())
-    assert len(ours) == len(theirs) == 22
-    for a, b in zip(ours, theirs):  # same directives, same arguments, same typed parameter sets
-        assert a[0] == b[0] and len(a) == len(b)
-        for x, y in zip(a[1:], b[1:]):
-            if isinstance(x, PS.ParamSet):
-                for bucket in PS.ParamSet.BUCKETS:
-                    dx, dy = getattr(x, bucket), getattr(y, bucket)
-                    assert dx.keys() == dy.keys() and all(np.array_equal(np.asarray(dx[k]), np.asarray(dy[k])) for k in dx), (a[0], bucket)
-            else:
-                assert np.array_equal(np.asarray(x), np.asarray(y)), a[0]
+def test_reference_spheres_scene_file_parses():
+    """The directives of the reference's src/scenes/spheres-differentials-texfilt.pbrt (directlighting "all", lowdiscrepancy sampler,
+    missing image map -> grey); tests/test_gpu_recursive_integrators.py renders the same file on the GPU."""
+    path = Path(__file__).parent / "golden" / "reference_spheres_scene.pbrt"
+    cmds = PP.parse_commands(path.read_text())
+    assert len(cmds) == 22 and cmds[-1] == ("WorldEnd",) and sum(c[0] == "WorldBegin" for c in cmds) == 1
     with warnings.catch_warnings():
         warnings.simplefilter("ignore")
-        job = pkg.pbrt_parse(REF_SCENES / "spheres-differentials-texfilt.pbrt").jobs[0]
+        job = pkg.pbrt_parse(path).jobs[0]
     assert job.integrator.kind == pkg.host.INTEGRATOR_DIRECT_ALL and len(job.flat.spheres) == 2 and job.flat.vertex_uv is not None
-    m = PLY.read_ply(str(REF_SCENES / "geometry" / "mesh_00001.ply"))  # the 88k-triangle caustic glass mesh
-    assert m["P"].shape == (44034, 3) and m["indices"].shape == (88064, 3) and m["N"].shape == (44034, 3)
-    # the same geometry with the path integrator: flattens, BVH builds, every triangle is referenced exactly once
-    # (its materials -- glass and uber -- are on the device path since round 2; only the sppm integrator is not)
-    text = (REF_SCENES / "caustic-glass.pbrt").read_text().replace('Integrator "sppm" "integer numiterations" [10000] "float radius" .075',
-                                                                   'Integrator "path" "integer maxdepth" [4]\nSampler "sobol" "integer pixelsamples" [1]')
-    with warnings.catch_warnings():
-        warnings.simplefilter("ignore")
-        job = pkg.pbrt_parse_string(text, search_dir=str(REF_SCENES)).jobs[0]
-    assert len(job.flat.tri_indices) == 88064 + 2 and len(job.flat.lights) == 2
-    assert job.flat.materials["type"].tolist() == [pkg.host.MAT_GLASS, pkg.host.MAT_UBER] and job.flat.materials["textured"].tolist() == [0, 1]
-    ext = job.flat.material_ext[1]
-    assert np.allclose(ext["s_const"][0], 0.64) and np.allclose(ext["s_const"][1], 0.1) and np.allclose(ext["s_const"][4], 1.0)
-    assert np.allclose(ext["f_const"], [0.010408, 0.010408, 1.0]) and len(job.flat.textures) == 0
-    # the oracle renders it (a 48-tile strip of the 700 x 1000 frame, 1 spp): finite, lit
-    from oracle import oracle as O
-    nt = job.integrator.n_tiles()
-    rgbw, st = O.render(job.flat, job.integrator, tile_range=(nt // 2, nt // 2 + 48))
-    assert np.isfinite(rgbw).all() and st["camera_rays"] > 10000 and rgbw[:, :3].sum() > 0
-    tri = job.flat.prims[job.flat.prims["shape_kind"] == pkg.host.SHAPE_TRIANGLE]
-    assert sorted(tri["shape_index"].tolist()) == list(range(88066))
-    assert job.film.full_resolution == (700, 1000) and job.film.scale == 1.5
