@@ -274,7 +274,9 @@ enum { PBRT_B200_INTEGRATOR_PATH = 0, PBRT_B200_INTEGRATOR_DIRECT_ONE = 1, PBRT_
 
 /* = PathIntegrator (src/integrators/path.rs:32-40,228-249); max_depth and pixel_bounds mean the same for
  * DirectLightingIntegrator (directlighting.rs:27-39,122-157) and WhittedIntegrator (whitted.rs), which ignore
- * rr_threshold and light_sample_strategy.                                                                  */
+ * rr_threshold and light_sample_strategy.  A negative max_depth means what path.rs's signed compare makes it:
+ * every path ends at its first hit.  Deviation from the reference, which has no upper bound: path and volpath
+ * reject max_depth > 65520 (PBRT_B200_ERR_INVALID), since the kernels count bounces in 16 bits.             */
 typedef struct pbrt_b200_integrator {
     int32_t  max_depth;
     float    rr_threshold;
@@ -462,7 +464,8 @@ typedef struct pbrt_b200_render_stats {
  * accumulates filter-weighted samples (FilmTile::add_sample, film.rs:292-331)
  * into rgbw_out[4 * width * height] over film.cropped_pixel_bounds as
  * {sum r, sum g, sum b, sum filter weight}; the buffer is ADDED to, so a caller
- * may split a render into several calls (or GPUs) and sum.  `stats` may be NULL. */
+ * may split a render into several calls (or GPUs) and sum.  `stats` may be NULL.
+ * Sample bounds wider or taller than 65535 pixels fail with PBRT_B200_ERR_INVALID. */
 int pbrt_b200_render(pbrt_b200_scene *scene, const pbrt_b200_render_desc *desc,
                      float *rgbw_out, pbrt_b200_render_stats *stats);
 

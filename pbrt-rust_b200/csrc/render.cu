@@ -2932,10 +2932,19 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
         if (zt) return fail(PBRT_B200_ERR_UNSUPPORTED, "render: volpath needs the sobol or halton sampler");
         if (rd->integrator.camera_medium < -1 || rd->integrator.camera_medium >= (int64_t)sc->dev.n_media)
             return fail(PBRT_B200_ERR_INVALID, "render: camera_medium out of range");
-        if (rd->integrator.max_depth > 0xfff0) return fail(PBRT_B200_ERR_INVALID, "render: volpath maxdepth too large");
     }
+    // the shade kernels keep the bounce count in 16 bits of the path state (volpath also counts down through material-less surfaces)
+    if (path_like && rd->integrator.max_depth > 0xfff0) return fail(PBRT_B200_ERR_INVALID, "render: path / volpath maxdepth above 65520");
     if (!path_like && (rd->integrator.max_depth < 1 || rd->integrator.max_depth > 64))
         return fail(PBRT_B200_ERR_INVALID, "render: directlighting / whitted need 1 <= maxdepth <= 64");
+    {   // path slots pack the pixel's offset in the sample bounds into 16 + 16 bits
+        const int* b = rd->sampler.sample_bounds;
+        if ((long long)b[2] - b[0] > 0xffff || (long long)b[3] - b[1] > 0xffff) {
+            char msg[160];
+            snprintf(msg, sizeof msg, "render: sample bounds [%d, %d) x [%d, %d) exceed 65535 pixels in x or y", b[0], b[2], b[1], b[3]);
+            return fail(PBRT_B200_ERR_INVALID, msg);
+        }
+    }
     PB_CUDA_TRY(cudaSetDevice(sc->device));
     int rc;
     DeviceShared* sh = device_shared(sc->device);
@@ -3045,7 +3054,8 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
     R.max_sample_luminance = rd->film.max_sample_luminance;
     R.filter_table = sh->filter_table;
     // integrator
-    R.max_depth = rd->integrator.max_depth; R.rr_threshold = rd->integrator.rr_threshold;
+    // the kernels compare the bounce count unsigned; path.rs compares signed, so a negative maxdepth ends every path at its first hit
+    R.max_depth = std::max(rd->integrator.max_depth, 0); R.rr_threshold = rd->integrator.rr_threshold;
     for (int i = 0; i < 4; ++i) R.pixel_bounds[i] = rd->integrator.pixel_bounds[i];
     R.ld_func = st->ld_func; R.ld_cdf = st->ld_cdf; R.ld_func_int = st->ld_func_int; R.n_lights = sc->dev.n_lights;
     R.inf_distrib = st->inf; R.infinite_lights = st->inf_list; R.n_infinite = st->n_inf;
@@ -3149,10 +3159,15 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
     R.u8 = nullptr;
     if (!zt && !R.rec.kind && !vol && S.kind == PBRT_B200_SAMPLER_SOBOL && S.log2_resolution > 0 && !getenv("PBRT_B200_NO_SOBOL_TABLES")) {
         const uint32_t sbw = (uint32_t)(sb[2] - sb[0]), sbh = (uint32_t)(sb[3] - sb[1]);
-        const uint32_t want = (uint32_t)std::min<long long>(1024, 5ll + 8ll * std::max(R.max_depth, 0));
+        // a path shading at bounce b < max_depth reads dimensions [s_dim, s_dim + 8) with s_dim <= 5 + 8b (camera 5, per bounce at most
+        // light choice 1 + light 2 + scattering 2 + BSDF 2 + roulette 1): the tables serve every block iff they hold 5 + 8 * max_depth dimensions
+        const unsigned long long dims_needed = 5ull + 8ull * (unsigned long long)R.max_depth;
+        const uint32_t want = (uint32_t)std::min<unsigned long long>(1024ull, dims_needed);
         uint32_t vdims = want;
         const size_t budget = (size_t)4 << 30;  // the pixel table may take up to 4 GB; deeper dimensions then go through k_sample_block
         while (vdims > 13u && (size_t)sbw * sbh * ((vdims + 3u) & ~3u) * 4u > budget) vdims -= 8u;
+        // test hook: fewer table dimensions, so that k_sample_block's table-index path runs on small films
+        if (const char* e = getenv("PBRT_B200_SOBOL_TABLE_DIMS")) vdims = std::min<uint32_t>(vdims, (uint32_t)std::max(1, atoi(e)));
         const uint32_t vstride = (vdims + 3u) & ~3u;
         const size_t vp_need = (size_t)sbw * sbh * vstride * 4u;
         const size_t vs_need = (size_t)std::max<uint32_t>(s_end - s_begin, 1u) * vstride * 4u;
@@ -3177,7 +3192,7 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
             if (ok) {
                 k_sobol_table_samples<<<64, 256, 0, stream>>>(T, sh->vs, s_begin, s_end - s_begin);
                 S.vp = sh->vp; S.vs = sh->vs; S.vdims = vdims; S.vstride = vstride; S.sbw = sbw; S.vs_begin = s_begin;
-                sample_prepass = vdims < want;
+                sample_prepass = dims_needed > vdims;  // paths past the tables' last block; beyond dimension 1024 too
             }
         }
     }
