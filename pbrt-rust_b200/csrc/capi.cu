@@ -62,6 +62,13 @@ __global__ void __launch_bounds__(PB_TRACE_BLOCK) k_intersect_batch(DevScene s, 
     BatchClosestJob job{rays, hits, s.tris};
     trace_queue<false, INST>(s, job, n, fetch, tune);
 }
+// Packet mode (trace.cuh: trace_queue_packet), scenes without instances, with PBRT_B200_PACKET_TRAVERSAL=2 only: a batch is
+// incoherent in general, so the batch API keeps the per-lane walk
+__global__ void __launch_bounds__(PB_TRACE_BLOCK) k_intersect_batch_packet(DevScene s, const float4* __restrict__ rays, uint32_t n, uint4* __restrict__ hits,
+                                                                          uint32_t* fetch) {
+    BatchClosestJob job{rays, hits, s.tris};
+    trace_queue_packet<false>(s, job, n, fetch);
+}
 
 // A/B variants for tuning (tools/trace_ab.py): one ray per thread, while-while or if-if
 template <int VARIANT>
@@ -82,6 +89,19 @@ __global__ void __launch_bounds__(PB_TRACE_BLOCK) k_intersect_p_batch(DevScene s
     BatchAnyJob job{rays, occluded};
     trace_queue<true, INST>(s, job, n, fetch);
 }
+__global__ void __launch_bounds__(PB_TRACE_BLOCK) k_intersect_p_batch_packet(DevScene s, const float4* __restrict__ rays, uint32_t n,
+                                                                            uint8_t* __restrict__ occluded, uint32_t* fetch) {
+    BatchAnyJob job{rays, occluded};
+    trace_queue_packet<true>(s, job, n, fetch);
+}
+
+namespace {
+// PBRT_B200_PACKET_TRAVERSAL=2 (read per call): the batch entry points walk aligned runs of 32 rays as packets
+bool batch_packet() {
+    const char* e = getenv("PBRT_B200_PACKET_TRAVERSAL");
+    return e && atoi(e) == 2;
+}
+}  // namespace
 
 // ---------------------------------------------------------------------------
 // scene
@@ -899,6 +919,9 @@ extern "C" int pbrt_b200_intersect_dev(pbrt_b200_scene* sc, const pbrt_b200_ray*
         if (sc->dev.n_instances)
             k_intersect_batch<true><<<grid, PB_TRACE_BLOCK, 0, (cudaStream_t)stream>>>(sc->dev, reinterpret_cast<const float4*>(rays), (uint32_t)n,
                                                                                        reinterpret_cast<uint4*>(hits), sc->fetch_counter, tune);
+        else if (batch_packet())
+            k_intersect_batch_packet<<<grid, PB_TRACE_BLOCK, 0, (cudaStream_t)stream>>>(sc->dev, reinterpret_cast<const float4*>(rays), (uint32_t)n,
+                                                                                        reinterpret_cast<uint4*>(hits), sc->fetch_counter);
         else
             k_intersect_batch<false><<<grid, PB_TRACE_BLOCK, 0, (cudaStream_t)stream>>>(sc->dev, reinterpret_cast<const float4*>(rays), (uint32_t)n,
                                                                                         reinterpret_cast<uint4*>(hits), sc->fetch_counter, tune);
@@ -918,6 +941,9 @@ extern "C" int pbrt_b200_intersect_p_dev(pbrt_b200_scene* sc, const pbrt_b200_ra
     if (sc->dev.n_instances)
         k_intersect_p_batch<true><<<sc->trace_grid, PB_TRACE_BLOCK, 0, (cudaStream_t)stream>>>(sc->dev, reinterpret_cast<const float4*>(rays), (uint32_t)n, occluded,
                                                                                               sc->fetch_counter);
+    else if (batch_packet())
+        k_intersect_p_batch_packet<<<sc->trace_grid, PB_TRACE_BLOCK, 0, (cudaStream_t)stream>>>(sc->dev, reinterpret_cast<const float4*>(rays), (uint32_t)n, occluded,
+                                                                                               sc->fetch_counter);
     else
         k_intersect_p_batch<false><<<sc->trace_grid, PB_TRACE_BLOCK, 0, (cudaStream_t)stream>>>(sc->dev, reinterpret_cast<const float4*>(rays), (uint32_t)n, occluded,
                                                                                                sc->fetch_counter);

@@ -913,6 +913,17 @@ __global__ void PB_TRACE_BOUNDS k_trace_closest(RenderDev R, int parity) {
     PathClosestJob job{&R, R.q_path[parity]};
     trace_queue<false, INST, PB_SH_STACK>(R.scene, job, R.cnt->n_path, &R.cnt->fetch_path, TraceTune{PB_WF_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN});
 }
+// Packet mode (trace.cuh: trace_queue_packet) for the camera rays of a wave's first iteration, scenes without instances.  A kernel of
+// its own: inside k_trace_closest<false> the packet walk took the per-lane kernel from 72 to 96 registers.  Left to itself ptxas gives
+// this one 96 registers (5 CTAs of 128 threads per SM); measured on S3 (B200, 64-spp step against 114.6-114.8 ms per-lane,
+// profiles/r03_packet_traversal.md): 5 CTAs 113.2 ms, 7 CTAs (71 registers) 111.4 ms, 8 CTAs (64 registers, 24 B of spills) 110.8 ms.
+#ifndef PB_TRACE_MINB_PACKET
+#define PB_TRACE_MINB_PACKET 8
+#endif
+__global__ void __launch_bounds__(PB_TRACE_BLOCK, PB_TRACE_MINB_PACKET) k_trace_closest_packet(RenderDev R, int parity) {
+    PathClosestJob job{&R, R.q_path[parity]};
+    trace_queue_packet<false, PB_SH_STACK>(R.scene, job, R.cnt->n_path, &R.cnt->fetch_path);
+}
 // Min resident CTAs per SM of the INSTANCED closest-hit / any-hit kernels (explicit specialisations: the plain kernels keep the compiler's
 // own choice, 72 registers; note that __launch_bounds__(n, 1) is NOT "no constraint" -- it lets ptxas take 126 registers there).  Left to
 // itself ptxas gives the two-level walk 96 / 80 registers = 5 / 6 CTAs of 128 threads; on S4 (gpurun_out/r2_s4_minb.log, 4-spp 4K step):
@@ -3131,6 +3142,9 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&shadow_per_sm, sc->dev.n_instances ? k_trace_shadow<true> : k_trace_shadow<false>, PB_TRACE_BLOCK, 0);
     cudaOccupancyMaxActiveBlocksPerMultiprocessor(&mis_per_sm, sc->dev.n_instances ? k_trace_mis<true> : k_trace_mis<false>, PB_TRACE_BLOCK, 0);
     int grid_shadow = sm_count * (shadow_per_sm > 0 ? shadow_per_sm : 1), grid_mis = sm_count * (mis_per_sm > 0 ? mis_per_sm : 1);
+    int packet_per_sm = 0;
+    cudaOccupancyMaxActiveBlocksPerMultiprocessor(&packet_per_sm, k_trace_closest_packet, PB_TRACE_BLOCK, 0);
+    const int grid_packet = sm_count * std::max(packet_per_sm, 1);
     // shade kernels keep 5 CTAs of 128 threads resident per SM (96-104 registers): 10 per SM = two full waves (8 left a
     // 3-CTA tail wave: -1.5 % on S3, gpurun_out/ab4.log)
     int grid_shade = sm_count * 20, grid_small = sm_count * 4;  // shade: 10 -> 20 CTAs per SM: 35.4 -> 35.2 ms per 16-spp S3 step (gpurun_out/r2o_grid.log)
@@ -3142,6 +3156,12 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
         grid_shadow = std::min(grid_shadow, need); grid_mis = std::min(grid_mis, need);
     }
 
+    // Packet traversal (trace.cuh: trace_queue_packet) for the closest-hit launch of a wave's first iteration: its queue holds the
+    // wave's camera rays in item order, so an aligned run of 32 is 32 samples of one pixel (samples innermost).  The later closest-hit,
+    // shadow and MIS queues lost with it on S3 (profiles/r03_packet_traversal.md) and keep the per-lane walk.
+    // PBRT_B200_PACKET_TRAVERSAL=0, read per call, turns it off (A/B on one build).
+    bool packet_camera = !zt;
+    if (const char* e = getenv("PBRT_B200_PACKET_TRAVERSAL")) if (atoi(e) == 0) packet_camera = false;
     cudaStream_t stream = 0;
     // events come from the scene's pool: [0] start, [1] end, [2..2+PB_PROG_RING) progress copies, then timing marks
     size_t ev_used = 2 + PB_PROG_RING;
@@ -3283,6 +3303,7 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
             launches += 3;
         }
         int parity = 0;
+        unsigned long long wave_iter = 0;  // iteration 0 traces the wave's camera rays
         const unsigned long long iter_cap = zt ? 256ull * spp_eff * (unsigned long long)(R.max_depth + 3) * 2ull + 4096
                                                : (total_items / capacity + 2) * (unsigned long long)(R.max_depth + 2 + 8) * 4ull *
                                                          (R.rec.kind ? 1ull << std::min(R.max_depth, 16) : 1ull) + 4096;  // recursive: a binary tree of rays
@@ -3292,6 +3313,7 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
             for (int b = 0; b < poll; ++b) {
                 if (timing) mark();
                 if (inst) k_trace_closest<true><<<grid_trace, PB_TRACE_BLOCK, 0, stream>>>(R, parity);
+                else if (packet_camera && wave_iter == 0) k_trace_closest_packet<<<grid_packet, PB_TRACE_BLOCK, 0, stream>>>(R, parity);
                 else k_trace_closest<false><<<grid_trace, PB_TRACE_BLOCK, 0, stream>>>(R, parity);
                 if (timing) mark();
                 if (R.sp.enabled && R.sp.lazy) {
@@ -3329,6 +3351,7 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
                 launches += 13;
                 parity ^= 1;
                 iter++;
+                wave_iter++;
             }
             // {item_cursor, n_path} of this batch -> ring entry, event marks the copy
             DeviceShared::Progress* pe = prog + (batch % PB_PROG_RING);

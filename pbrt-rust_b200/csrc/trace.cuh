@@ -577,11 +577,15 @@ PB_D void trav_run_impl(const DevScene& s, TravRay& r, STK stack, int yield_belo
 // slot inside each group by the child's axis), later ones are stacked behind earlier ones, and a stacked entry is
 // re-checked against the current t_max when popped, as in the binary walk.  Only for rays without zero direction
 // components (slab_fast's precondition; the others take the binary, NaN-exact walk).
-template <bool ANY, typename STK>
-PB_D void quad_step(const DevScene& s, TravRay& r, STK stack) {
+//
+// quad_slots: the four slots of quad node `node` in visiting order -- t[k] = the slot's tmin (+inf when its slab test fails), ref[k]
+// its reference.  The order depends on the ray only through `negmask` (trav_run_packet passes its warp's shared octant, which
+// makes ref[] warp-uniform).
+template <bool ANY>
+PB_D void quad_slots(const DevScene& s, const TravRay& r, uint32_t node, uint32_t negmask, float* t, uint32_t* ref) {
 #if PB_CQUAD
     // {lower corner, ex | ey << 8 | ez << 16 | meta << 24}, {refs}, {lo.x[4], lo.y[4], lo.z[4], hi.x[4]}, {hi.y[4], hi.z[4], -, -}
-    const float4* np = s.cquads + 4ull * r.cur;
+    const float4* np = s.cquads + 4ull * node;
     const float4 hd = __ldg(np), q6 = __ldg(np + 1), qa = __ldg(np + 2), qb = __ldg(np + 3);
     const uint32_t hb = __float_as_uint(hd.w);
     // plane = corner + q * 2^e  ->  t = q * (2^e / d) + (corner - o) / d : one FFMA per plane (f32x2: two children per issue slot)
@@ -628,7 +632,7 @@ PB_D void quad_step(const DevScene& s, TravRay& r, STK stack) {
 #undef PB_Q23
     const float4 q7 = make_float4(__uint_as_float(hb >> 24), 0.0f, 0.0f, 0.0f);
 #else
-    const float4* np = s.quads + 8ull * r.cur;
+    const float4* np = s.quads + 8ull * node;
     const float4 a0 = __ldg(np), a1 = __ldg(np + 1), a2 = __ldg(np + 2), b0 = __ldg(np + 3), b1 = __ldg(np + 4), b2 = __ldg(np + 5), q6 = __ldg(np + 6), q7 = __ldg(np + 7);
     SlabPair pa = slab_fast2(r.ngx ? make_float2(a1.z, a1.w) : make_float2(a0.x, a0.y), r.ngy ? make_float2(a2.x, a2.y) : make_float2(a0.z, a0.w),
                              r.ngz ? make_float2(a2.z, a2.w) : make_float2(a1.x, a1.y), r.ngx ? make_float2(a0.x, a0.y) : make_float2(a1.z, a1.w),
@@ -641,7 +645,7 @@ PB_D void quad_step(const DevScene& s, TravRay& r, STK stack) {
 #endif
     const float tA0 = pa.ok0 ? pa.tmin0 : PB_INF, tA1 = pa.ok1 ? pa.tmin1 : PB_INF, tB0 = pb.ok0 ? pb.tmin0 : PB_INF, tB1 = pb.ok1 ? pb.tmin1 : PB_INF;
     const uint32_t meta = __float_as_uint(q7.x);
-    const bool g = (r.negmask >> (meta & 3u)) & 1u, sA = (r.negmask >> ((meta >> 2) & 3u)) & 1u, sB = (r.negmask >> ((meta >> 4) & 3u)) & 1u;
+    const bool g = (negmask >> (meta & 3u)) & 1u, sA = (negmask >> ((meta >> 2) & 3u)) & 1u, sB = (negmask >> ((meta >> 4) & 3u)) & 1u;
     // reference order inside each group, then of the groups
     const float tAn = sA ? tA1 : tA0, tAf = sA ? tA0 : tA1, tBn = sB ? tB1 : tB0, tBf = sB ? tB0 : tB1;
     const uint32_t rAn = __float_as_uint(sA ? q6.y : q6.x), rAf = __float_as_uint(sA ? q6.x : q6.y);
@@ -655,6 +659,16 @@ PB_D void quad_step(const DevScene& s, TravRay& r, STK stack) {
     const float t0 = g ? tBn : tAn, t1 = g ? tBf : tAf, t2 = g ? tAn : tBn, t3 = g ? tAf : tBf;
     const uint32_t r0 = g ? rBn : rAn, r1 = g ? rBf : rAf, r2 = g ? rAn : rBn, r3 = g ? rAf : rBf;
 #endif
+    t[0] = t0; t[1] = t1; t[2] = t2; t[3] = t3;
+    ref[0] = r0; ref[1] = r1; ref[2] = r2; ref[3] = r3;
+}
+template <bool ANY, typename STK>
+PB_D void quad_step(const DevScene& s, TravRay& r, STK stack) {
+    float t[4];
+    uint32_t ref[4];
+    quad_slots<ANY>(s, r, r.cur, r.negmask, t, ref);
+    const float t0 = t[0], t1 = t[1], t2 = t[2], t3 = t[3];
+    const uint32_t r0 = ref[0], r1 = ref[1], r2 = ref[2], r3 = ref[3];
     // the first slot that passes is visited now; the others wait on the stack, nearest on top
     uint32_t nref = PB_DONE; float ntm = 0.0f;
 #if PB_PREFETCH_FAR
@@ -783,6 +797,63 @@ PB_D void trav_run_quad_coop(const DevScene& s, TravRay& r, STK stack, int yield
         const int alive = __popc(__ballot_sync(FULL, !trav_done(r)));
         if (alive == 0 || alive < yield_below) break;
     }
+}
+
+// PACKET form: ALL 32 lanes call it together and share ONE depth-first walk over the union of the nodes their rays need, so every
+// lane is on the same node or leaf at every step and each node / leaf fetch is one broadcast load.  Precondition: every lane that
+// has a ray (r.cur != PB_DONE after trav_init) has no zero direction component and the octant `negmask` (trace_queue_packet checks
+// it).  The stack is the lanes' own stack at a warp-uniform depth: every lane writes the entry's (warp-uniform) node reference with
+// ITS tmin for that slot, or +inf when it does not pass the slot, and a pop's lane mask is the ballot of `tmin < t_max` -- the
+// per-lane walk's own pop test.
+// Exactness: quad_slots orders the slots by the shared octant, so each lane meets the nodes it passes in the order the per-lane
+// walk would (depth-first, near slot first), and a node's mask only holds lanes that passed it.  A slot a lane passes but the warp
+// does not visit first waits on the stack behind slots that lane failed; the lane is idle in their sub-trees, so its t_max has not
+// changed when the slot is popped and the pop's re-check passes, as the direct visit would have.  Each lane thus runs the same box
+// and primitive tests, in the same order, against the same t_max as alone: same tie-breaks, bit-identical hits.
+template <bool ANY, typename STK>
+PB_D void trav_run_packet(const DevScene& s, TravRay& r, STK stack, uint32_t negmask) {
+    const unsigned FULL = 0xffffffffu, lane_bit = 1u << (threadIdx.x & 31u);
+    uint32_t mask = __ballot_sync(FULL, r.cur != PB_DONE);  // lanes whose ray passed the root box
+    uint32_t cur = mask ? s.root_ref : PB_DONE;
+    int sp = 0;  // warp-uniform
+#define PB_PACKET_POP()                                                              \
+    do {                                                                             \
+        cur = PB_DONE;                                                               \
+        while (sp > 0) {                                                             \
+            --sp;                                                                    \
+            const uint2 e__ = stack.get(sp);                                         \
+            mask = __ballot_sync(FULL, __uint_as_float(e__.y) < r.t_max);            \
+            if (mask) { cur = e__.x; break; }                                        \
+        }                                                                            \
+    } while (0)
+    while (cur != PB_DONE) {
+        while (!(cur & PB_LEAF_BIT)) {
+            const bool live = mask & lane_bit;
+            float t[4];
+            uint32_t ref[4];
+            quad_slots<ANY>(s, r, cur, negmask, t, ref);
+            // the first slot any lane passes is visited now; the others wait on the stack, nearest on top
+            uint32_t nref = PB_DONE, nmask = 0;
+            float ntm = PB_INF;
+#pragma unroll
+            for (int k = 3; k >= 0; --k) {
+                const bool p = live && t[k] < r.t_max;
+                const uint32_t m = __ballot_sync(FULL, p);
+                if (m) {
+                    if (nref != PB_DONE) { stack.put(sp, make_uint2(nref, __float_as_uint(ntm))); ++sp; }
+                    nref = ref[k]; nmask = m; ntm = p ? t[k] : PB_INF;
+                }
+            }
+            cur = nref; mask = nmask;
+            if (cur == PB_DONE) PB_PACKET_POP();
+        }
+        if (cur == PB_DONE) break;
+        // an any-hit lane that found an occluder is finished: t_max = -inf fails every later pop
+        if ((mask & lane_bit) && quad_leaf_run<ANY>(s, r, cur & ~PB_LEAF_BIT)) r.t_max = -PB_INF;
+        PB_PACKET_POP();
+    }
+#undef PB_PACKET_POP
+    r.cur = PB_DONE; r.sp = 0;
 }
 
 // INST: the scene contains TransformedPrimitives.  Scenes without instancing run kernels compiled with INST = false, which
@@ -925,11 +996,16 @@ PB_D bool traverse_ifif(const DevScene& s, f3 o, f3 d, float t_max, RayHit* hit)
 #define PB_INTERIOR_MIN 16
 #endif
 struct TraceTune { int refill_below; int chunk; int interior_min; };
+// The shared levels of the hybrid stack: one array per kernel, which trace_queue and trace_queue_packet both use.
+template <int SH>
+PB_D uint2* trace_stack_shared() {
+    __shared__ uint2 stack_shared[SH > 0 ? SH : 1][PB_TRACE_BLOCK];
+    return &stack_shared[0][threadIdx.x];
+}
 template <bool ANY, bool INST, int SH = 0, typename Job>
 PB_D void trace_queue(const DevScene& s, Job& job, uint32_t n, uint32_t* fetch_counter, TraceTune tune = TraceTune{PB_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN}) {
     uint2 stack_mem[PB_STACK_SIZE(INST)];
-    __shared__ uint2 stack_shared[SH > 0 ? SH : 1][PB_TRACE_BLOCK];
-    HybridStack<SH, PB_TRACE_BLOCK> stack{&stack_shared[0][threadIdx.x], stack_mem};  // SH == 0: every level in the local array
+    HybridStack<SH, PB_TRACE_BLOCK> stack{trace_stack_shared<SH>(), stack_mem};  // SH == 0: every level in the local array
     TravRay r;
     r.cur = PB_DONE; r.pend = PB_DONE; r.sp = 0; r.found = false;
     uint32_t ray_idx = 0xffffffffu;
@@ -985,6 +1061,40 @@ PB_D void trace_queue(const DevScene& s, Job& job, uint32_t n, uint32_t* fetch_c
         }
 #endif
         trav_run<ANY, INST>(s, r, stack, exhausted ? 0 : tune.refill_below, tune.interior_min);
+    }
+}
+
+// Packet mode of the ray queue (scenes without instances), for queues whose aligned runs of 32 entries are coherent rays: camera
+// rays in item order (32 samples of one pixel) and the shadow rays cast from their hits.  A warp takes a whole aligned chunk of 32
+// entries -- lane-wise refills would mix pixels -- and walks it as one packet (trav_run_packet) when all its rays share an octant
+// and have no zero direction component; any other chunk runs the per-lane walk to completion.
+template <bool ANY, int SH = 0, typename Job>
+PB_D void trace_queue_packet(const DevScene& s, Job& job, uint32_t n, uint32_t* fetch_counter) {
+    uint2 stack_mem[PB_STACK_SIZE(false)];
+    HybridStack<SH, PB_TRACE_BLOCK> stack{trace_stack_shared<SH>(), stack_mem};
+    const unsigned FULL = 0xffffffffu, lane = threadIdx.x & 31u;
+    for (;;) {
+        uint32_t b = 0;
+        if (lane == 0) b = atomicAdd(fetch_counter, 32u);
+        b = __shfl_sync(FULL, b, 0);
+        if (b >= n) break;
+        const uint32_t idx = b + lane;
+        TravRay r;
+        r.cur = PB_DONE; r.pend = PB_DONE; r.sp = 0; r.found = false;
+        r.hit.slot = PBRT_B200_NO_HIT; r.hit.inst = PBRT_B200_NO_HIT;
+        f3 o, d; float t_max = 0.0f;
+        if (idx < n) {
+            if (job.load(idx, &o, &d, &t_max)) trav_init(s, r, o, d, t_max);
+            else r.hit.t = t_max;
+        }
+        // octant of the chunk: the first lane that traverses; 8 = a zero direction component, never shared
+        const bool trav = r.cur != PB_DONE;
+        const uint32_t oct = trav ? (r.nan_possible ? 8u : r.negmask) : 0u;
+        const uint32_t first = __ffs(__ballot_sync(FULL, trav));
+        const uint32_t shared_oct = __shfl_sync(FULL, oct, first ? first - 1 : 0);
+        if (__all_sync(FULL, !trav || oct == shared_oct) && shared_oct != 8u) trav_run_packet<ANY>(s, r, stack, shared_oct);
+        else if (trav) trav_run<ANY, false>(s, r, stack, 0);
+        if (idx < n) job.store(idx, r);
     }
 }
 
