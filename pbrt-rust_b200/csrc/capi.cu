@@ -270,61 +270,6 @@ __global__ void __launch_bounds__(256) k_quad_nodes(const float4* __restrict__ f
     }
 }
 
-#if PB_CQUAD
-// quad nodes -> compressed quad nodes (A/B, trace.cuh PB_CQUAD): per node a lower corner and one power-of-two grid step per axis; a child plane is a
-// byte on that grid, rounded outward and then given one more quantum of slack, so that the decoded box contains the exact one with a margin far above
-// the rounding of the ray-space decode.  Empty slots are recognised by their ref.
-__global__ void __launch_bounds__(256) k_cquad_nodes(const float4* __restrict__ quads, uint32_t n_fat, float4* __restrict__ cq) {
-    for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < n_fat; i += gridDim.x * blockDim.x) {
-        const float4* q = quads + 8ull * i;
-        float lo[4][3], hi[4][3];
-        for (int pr = 0; pr < 2; ++pr) {
-            const float4 c0 = q[3 * pr], c1 = q[3 * pr + 1], c2 = q[3 * pr + 2];
-            const int a = 2 * pr, b = 2 * pr + 1;
-            lo[a][0] = c0.x; lo[b][0] = c0.y; lo[a][1] = c0.z; lo[b][1] = c0.w; lo[a][2] = c1.x; lo[b][2] = c1.y;
-            hi[a][0] = c1.z; hi[b][0] = c1.w; hi[a][1] = c2.x; hi[b][1] = c2.y; hi[a][2] = c2.z; hi[b][2] = c2.w;
-        }
-        const float4 refs = q[6];
-        const uint32_t ref[4] = {__float_as_uint(refs.x), __float_as_uint(refs.y), __float_as_uint(refs.z), __float_as_uint(refs.w)};
-        float corner[3];
-        uint32_t ebits = 0, wlo[3] = {0, 0, 0}, whi[3] = {0, 0, 0};
-        for (int a = 0; a < 3; ++a) {
-            float mn = __int_as_float(0x7f800000), mx = -mn;
-            for (int c = 0; c < 4; ++c)
-                if (ref[c] != PB_REF_NONE) { mn = fminf(mn, lo[c][a]); mx = fmaxf(mx, hi[c][a]); }
-            corner[a] = mn;
-            int e;
-            frexpf(fmaxf(mx - mn, 1e-30f) / 253.0f, &e);  // 2^e > extent / 253
-            uint32_t ql[4], qh[4];
-            for (;; ++e) {
-                const float s = ldexpf(1.0f, e);
-                bool fits = true;
-                for (int c = 0; c < 4 && fits; ++c) {
-                    if (ref[c] == PB_REF_NONE) { ql[c] = 255; qh[c] = 0; continue; }
-                    int l = (int)floorf((lo[c][a] - mn) / s), h = (int)ceilf((hi[c][a] - mn) / s);
-                    while (l > 0 && __fmaf_rn((float)l, s, mn) > lo[c][a]) --l;
-                    while (h < 300 && __fmaf_rn((float)h, s, mn) < hi[c][a]) ++h;
-                    l = l > 0 ? l - 1 : 0; h += 1;  // one quantum of slack
-                    if (h > 255) fits = false;
-                    ql[c] = (uint32_t)l; qh[c] = (uint32_t)h;
-                }
-                if (fits) break;
-            }
-            e = e < -125 ? -125 : e;  // (never reached by real scenes: extents below 1e-30)
-            ebits |= (uint32_t)(e + 127) << (8 * a);
-            wlo[a] = ql[0] | (ql[1] << 8) | (ql[2] << 16) | (ql[3] << 24);
-            whi[a] = qh[0] | (qh[1] << 8) | (qh[2] << 16) | (qh[3] << 24);
-        }
-        const uint32_t meta = __float_as_uint(q[7].x) & 0x3fu;
-        float4* o = cq + 4ull * i;
-        o[0] = make_float4(corner[0], corner[1], corner[2], __uint_as_float(ebits | (meta << 24)));
-        o[1] = refs;
-        o[2] = make_float4(__uint_as_float(wlo[0]), __uint_as_float(wlo[1]), __uint_as_float(wlo[2]), __uint_as_float(whi[0]));
-        o[3] = make_float4(__uint_as_float(whi[1]), __uint_as_float(whi[2]), 0.0f, 0.0f);
-    }
-}
-#endif
-
 __global__ void k_single_prim_last(const uint32_t* __restrict__ slots, uint32_t n, float4* __restrict__ tris) {
     for (uint32_t k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) {
         float4* rec = tris + 3ull * slots[k] + 1;
@@ -701,9 +646,6 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
     size_t need = 0;
     auto add = [&](size_t bytes) { need += Arena::padded(bytes); };
     add(64ull * max_interior); add(128ull * max_interior); add(48ull * np); add(sizeof(pbrt_b200_prim) * np);
-#if PB_CQUAD
-    add(64ull * max_interior);
-#endif
     add(12ull * nv); add(d->vertex_n ? 12ull * nv : 0); add(d->vertex_s ? 12ull * nv : 0); add(d->vertex_uv ? 8ull * nv : 0);
     add(12ull * nt); add(sizeof(pbrt_b200_sphere) * d->n_spheres); add(sizeof(pbrt_b200_material) * d->n_materials); add(sizeof(pbrt_b200_light) * d->n_lights);
     add(sizeof(DevInstance) * d->n_instances); add(4ull * d->n_objects); add(sizeof(DevScene));
@@ -760,10 +702,6 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
     float4* quads = A.take<float4>(8ull * max_interior);
     float4* tris = A.take<float4>(3ull * np);
     ds.nodes = fat; ds.quads = quads; ds.tris = tris;
-#if PB_CQUAD
-    float4* cquads = A.take<float4>(4ull * max_interior);
-    ds.cquads = cquads;
-#endif
     float4* slot_n = (d->vertex_n && np) ? A.take<float4>(3ull * np) : nullptr;
     float2* slot_uv = (d->vertex_uv && np) ? A.take<float2>(3ull * np) : nullptr;
     float4* light_tris = d->n_lights ? A.take<float4>(6ull * d->n_lights) : nullptr;
@@ -822,9 +760,6 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
             fat_launch(0, d->n_objects ? d->n_top_nodes : nn, 0);
             for (uint64_t k = 0; k < d->n_objects; ++k) fat_launch(d->objects[k].node_offset, d->objects[k].n_nodes, d->objects[k].prim_offset);
             if (n_interior) k_quad_nodes<<<(unsigned)std::min<uint64_t>((n_interior + 255) / 256, 148 * 16), 256, 0, stream>>>(fat, n_interior, quads);
-#if PB_CQUAD
-            if (n_interior) k_cquad_nodes<<<(unsigned)std::min<uint64_t>((n_interior + 255) / 256, 148 * 16), 256, 0, stream>>>(quads, n_interior, cquads);
-#endif
         }
     }
     if (d->n_instances && err == cudaSuccess) {

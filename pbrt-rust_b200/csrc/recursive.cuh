@@ -161,17 +161,17 @@ PB_D void rec_estimate_direct(const RenderDev& R, uint32_t id, const Surf& si, c
 // (compute_scattering_functions always runs compute_differentials, interaction.rs:258-267), and specular_reflect / specular_transmit
 // hand differentials on to the rays they spawn (integrator.rs:427-452, 476-513).
 template <bool INST, bool ZT, bool TEX>
-__global__ void __launch_bounds__(PB_REC_LOCKSTEP || TEX ? PB_REC_TEX_BLOCK : 128) k_rec_shade(RenderDev R, int parity) {
+__global__ void __launch_bounds__(PB_REC_BLOCK) k_rec_shade(RenderDev R, int parity) {
     constexpr int KM = TEX ? KM_TEX : KM_ALL;
     const uint32_t n = R.cnt->n_path;
     const uint32_t* q = R.q_path[parity];
     uint32_t* q_next = R.q_path[parity ^ 1];
-    // TEX: 56 k instructions (the texture interpreter on top of every BSDF and the recursion frames) -- as k_shade<Q_TEX>, the CTA is the whole
-    // SM and its warps start every path behind a barrier, so that they stay close to each other in the code (instruction cache)
-    const uint32_t nround = (PB_REC_LOCKSTEP || TEX) ? ((n + blockDim.x - 1u) / blockDim.x) * blockDim.x : ((n + 31u) & ~31u);
+    // 35 k instructions (TEX: 56 k, the texture interpreter on top of every BSDF and the recursion frames) -- as k_shade<Q_TEX>, the CTA is
+    // the whole SM and its warps start every path behind a barrier, so that they stay close to each other in the code (instruction cache)
+    const uint32_t nround = ((n + blockDim.x - 1u) / blockDim.x) * blockDim.x;
     const uint32_t D = R.rec.stack_depth;
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < nround; i += gridDim.x * blockDim.x) {
-        if (PB_REC_LOCKSTEP || TEX) __syncthreads();
+        __syncthreads();
         bool push_next = false, push_dead = false;
         uint32_t id = 0;
         if (i < n) {
@@ -401,7 +401,7 @@ struct RecShadowJob {
     }
 };
 template <bool INST>
-__global__ void PB_TRACE_BOUNDS k_rec_shadow(RenderDev R) {
+__global__ void __launch_bounds__(PB_TRACE_BLOCK) k_rec_shadow(RenderDev R) {
     RecShadowJob job{&R};
     trace_queue<true, INST, PB_SH_STACK>(R.scene, job, R.cnt->n_shadow, &R.cnt->fetch_shadow);
 }
@@ -434,7 +434,7 @@ struct RecMisJob {
     }
 };
 template <bool INST>
-__global__ void PB_TRACE_BOUNDS k_rec_mis(RenderDev R) {
+__global__ void __launch_bounds__(PB_TRACE_BLOCK) k_rec_mis(RenderDev R) {
     RecMisJob<INST> job{&R};
     trace_queue<false, INST, PB_SH_STACK>(R.scene, job, R.cnt->n_mis, &R.cnt->fetch_mis);
 }

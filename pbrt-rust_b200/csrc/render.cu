@@ -28,27 +28,11 @@
 #include "texture.cuh"
 #include "util.cuh"
 
-// occupancy knobs (min resident CTAs per SM in __launch_bounds__), A/B-measured with tools/step_diag.py on S3: shade 5/6/8 CTAs
-// (96/80/64 registers) and trace 6/8/10 CTAs are all within +-1% or slower than the compiler's default choice
-#ifdef PB_SHADE_MINB
-#define PB_SHADE_BOUNDS __launch_bounds__(128, PB_SHADE_MINB)
-#else
-#define PB_SHADE_BOUNDS __launch_bounds__(BIN == Q_TEX ? PB_TEX_BLOCK : 128)
-#endif
-#ifndef PB_REC_LOCKSTEP
-#define PB_REC_LOCKSTEP 1  /* the plain k_rec_shade kernels (35 k instructions, 168 registers) phase-locked like the textured one */
-#endif
-#ifndef PB_REC_TEX_BLOCK
-#define PB_REC_TEX_BLOCK 384  /* threads per CTA of k_rec_shade<.., TEX> (168 registers: one CTA per SM) */
-#endif
-#ifndef PB_TEX_BLOCK
+// Min resident CTAs per SM in __launch_bounds__, A/B-measured with tools/step_diag.py on S3: shade 5/6/8 CTAs (96/80/64 registers) and
+// trace 6/8/10 CTAs are all within +-1% or slower than the compiler's default choice, so the shade kernels and the plain trace kernels
+// set none.
+#define PB_REC_BLOCK 384  /* threads per CTA of k_rec_shade (168 registers: one CTA per SM whose warps start every path together, see the kernel) */
 #define PB_TEX_BLOCK 512  /* threads per CTA of k_shade<Q_TEX>: one CTA per SM whose warps start every path together (see k_shade) */
-#endif
-#ifdef PB_TRACE_MINB
-#define PB_TRACE_BOUNDS __launch_bounds__(PB_TRACE_BLOCK, PB_TRACE_MINB)
-#else
-#define PB_TRACE_BOUNDS __launch_bounds__(PB_TRACE_BLOCK)
-#endif
 
 // This file is compiled THREE times (csrc/Makefile; mega.o -- the one-kernel forms -- is described where PB_MEGA_TU is defined below):
 //   render.o  (PB_EXACT_TU = 1, --fmad=false, IEEE division / square root): ray generation, traversal, film, light tables, the
@@ -60,12 +44,7 @@
 // Refill threshold of the wavefront trace kernels (lanes whose ray has finished are refilled once fewer than this many are still
 // traversing).  Swept at 64 spp with runtime knobs (gpurun_out/r2q_tune.log): 16 -> 132.4 ms per step, 20 -> 133.2, 24 -> 134.7, 28 -> 136.5,
 // 32 -> 141.0; interior_min 16 stays the best of 0 / 8 / 12 / 16 / 20 / 24.  (Compile-time constants: the runtime knobs cost 3 %.)
-#ifndef PB_WF_REFILL_BELOW
 #define PB_WF_REFILL_BELOW 16
-#endif
-#ifndef PB_SAMPLES_INNER
-#define PB_SAMPLES_INNER 1
-#endif
 // Three translation units from this one source (csrc/Makefile): render.o (PB_EXACT_TU: everything but the kernels below, host side
 // included), shade.o (PB_TU_SHADE, --use_fast_math: k_shade / k_rec_shade) and mega.o (PB_TU_MEGA, exact flags: the one-kernel forms
 // k_zt_mega / k_vol_mega, whose out-of-line shade bodies are 2 minutes of ptxas on their own -- a separate unit compiles in parallel).
@@ -80,12 +59,8 @@
 #define PB_MEGA_TU 0
 #endif
 #define PB_SHADE_TU (!PB_EXACT_TU && !PB_MEGA_TU)
-#ifndef PB_ZT_WARPS
 #define PB_ZT_WARPS 4u    /* warps per CTA of k_zt_mega (the host aims at ~4 warps per SM: one CTA), phases of a trip passed together */
-#endif
-#ifndef PB_VOL_BLOCK
-#define PB_VOL_BLOCK 512  /* threads per CTA of k_vol_mega.  > 64: the CTA's warps pass the phases of a trip together (barriers between them): see the kernel */
-#endif
+#define PB_VOL_BLOCK 512  /* threads per CTA of k_vol_mega: the CTA's warps pass the phases of a trip together (barriers between them): see the kernel */
 
 using namespace pb;
 
@@ -768,7 +743,7 @@ PB_D bool tile_xy(const RenderDev& R, uint32_t t, int* tx, int* ty) {
 }
 
 // One camera sample into path slot `slot`.  Returns false when the item falls outside the sample/pixel bounds (partial edge
-// tiles) -- the slot then stays free.  Item order (PB_SAMPLES_INNER): (tile, pixel-in-tile, sample) with the samples of the call
+// tiles) -- the slot then stays free.  Item order: (tile, pixel-in-tile, sample) with the samples of the call
 // INNERMOST, so the 32 lanes of a warp carry consecutive samples of ONE pixel (when the call has >= 32 of them): their camera
 // rays walk the same nodes (one L1 wavefront per load instead of one per lane), hit the same few triangles, read the same pixel row
 // of the sampler table, and their film contributions collapse into one atomic per warp.  The alternative (samples outermost:
@@ -776,23 +751,12 @@ PB_D bool tile_xy(const RenderDev& R, uint32_t t, int* tx, int* ty) {
 // number), so the image does not depend on the order (only the film's f32 summation order does).
 PB_D bool gen_camera_path(const RenderDev& R, unsigned long long item, uint32_t slot) {
     uint32_t p, j, sample;  // pixel in tile; ordinal among the tiles this call owns; sample number
-#if PB_SAMPLES_INNER
     {
         unsigned long long pp;  // tile-pixel ordinal
         if ((item >> 32) == 0) { const uint32_t i32 = (uint32_t)item, q = i32 / R.n_samples_sel; sample = i32 - q * R.n_samples_sel + R.sample_begin; pp = q; }
         else { pp = item / R.n_samples_sel; sample = (uint32_t)(item - pp * R.n_samples_sel) + R.sample_begin; }
         p = (uint32_t)(pp & 255u); j = (uint32_t)(pp >> 8);
     }
-#else
-    p = (uint32_t)(item & 255u);
-    unsigned long long rest = item >> 8;
-    if ((rest >> 32) == 0) {  // (always, short of 2^40 items in one call): one 32-bit division instead of two emulated 64-bit ones
-        const uint32_t r32 = (uint32_t)rest, qs = r32 / R.n_tiles_sel;
-        j = r32 - qs * R.n_tiles_sel; sample = qs + R.sample_begin;
-    } else {
-        j = (uint32_t)(rest % R.n_tiles_sel); sample = (uint32_t)(rest / R.n_tiles_sel) + R.sample_begin;
-    }
-#endif
     const uint32_t jg = j / R.tile_group;
     uint32_t t = R.tile_begin + (jg * R.tile_mod + R.tile_rem) * R.tile_group + (j - jg * R.tile_group);
     int tx, ty;
@@ -909,7 +873,7 @@ struct PathClosestJob {
 };
 
 template <bool INST>
-__global__ void PB_TRACE_BOUNDS k_trace_closest(RenderDev R, int parity) {
+__global__ void __launch_bounds__(PB_TRACE_BLOCK) k_trace_closest(RenderDev R, int parity) {
     PathClosestJob job{&R, R.q_path[parity]};
     trace_queue<false, INST, PB_SH_STACK>(R.scene, job, R.cnt->n_path, &R.cnt->fetch_path, TraceTune{PB_WF_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN});
 }
@@ -917,9 +881,7 @@ __global__ void PB_TRACE_BOUNDS k_trace_closest(RenderDev R, int parity) {
 // its own: inside k_trace_closest<false> the packet walk took the per-lane kernel from 72 to 96 registers.  Left to itself ptxas gives
 // this one 96 registers (5 CTAs of 128 threads per SM); measured on S3 (B200, 64-spp step against 114.6-114.8 ms per-lane,
 // profiles/r03_packet_traversal.md): 5 CTAs 113.2 ms, 7 CTAs (71 registers) 111.4 ms, 8 CTAs (64 registers, 24 B of spills) 110.8 ms.
-#ifndef PB_TRACE_MINB_PACKET
 #define PB_TRACE_MINB_PACKET 8
-#endif
 __global__ void __launch_bounds__(PB_TRACE_BLOCK, PB_TRACE_MINB_PACKET) k_trace_closest_packet(RenderDev R, int parity) {
     PathClosestJob job{&R, R.q_path[parity]};
     trace_queue_packet<false, PB_SH_STACK>(R.scene, job, R.cnt->n_path, &R.cnt->fetch_path);
@@ -928,26 +890,13 @@ __global__ void __launch_bounds__(PB_TRACE_BLOCK, PB_TRACE_MINB_PACKET) k_trace_
 // own choice, 72 registers; note that __launch_bounds__(n, 1) is NOT "no constraint" -- it lets ptxas take 126 registers there).  Left to
 // itself ptxas gives the two-level walk 96 / 80 registers = 5 / 6 CTAs of 128 threads; on S4 (gpurun_out/r2_s4_minb.log, 4-spp 4K step):
 // default 303.9 ms, 6 CTAs (80 regs, closest only) 288.8, 7 CTAs (72 regs, both, 6-92 B of spills) 285.2, 8 CTAs (64 regs) 309.6.
-#ifndef PB_TRACE_MINB_INST
 #define PB_TRACE_MINB_INST 7
-#endif
-#ifndef PB_TRACE_MINB_INST_ANY
 #define PB_TRACE_MINB_INST_ANY 7
-#endif
-#ifdef PB_TRACE_MINB_PLAIN  /* A/B knob: the plain closest-hit kernel alone */
-template <>
-__global__ void __launch_bounds__(PB_TRACE_BLOCK, PB_TRACE_MINB_PLAIN) k_trace_closest<false>(RenderDev R, int parity) {
-    PathClosestJob job{&R, R.q_path[parity]};
-    trace_queue<false, false, PB_SH_STACK>(R.scene, job, R.cnt->n_path, &R.cnt->fetch_path, TraceTune{PB_WF_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN});
-}
-#endif
-#if PB_TRACE_MINB_INST > 0
 template <>
 __global__ void __launch_bounds__(PB_TRACE_BLOCK, PB_TRACE_MINB_INST) k_trace_closest<true>(RenderDev R, int parity) {
     PathClosestJob job{&R, R.q_path[parity]};
     trace_queue<false, true, PB_SH_STACK>(R.scene, job, R.cnt->n_path, &R.cnt->fetch_path, TraceTune{PB_WF_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN});
 }
-#endif
 
 // sort/compact-by-material.  Lanes of the same bin form a group (match.any) and the groups of the CTA's eight warps are
 // added up in shared memory: one atomicAdd per bin per 256 paths (the per-warp form waited on the atomic's round trip for 83 % of
@@ -1641,7 +1590,7 @@ PB_D ShadeOut shade_path(const RenderDev& R, uint32_t id, VolState* vs = nullptr
 
 #if PB_SHADE_TU
 template <int BIN, bool INST, bool ZT>
-__global__ void PB_SHADE_BOUNDS k_shade(RenderDev R, int parity) {
+__global__ void __launch_bounds__(BIN == Q_TEX ? PB_TEX_BLOCK : 128) k_shade(RenderDev R, int parity) {
     const uint32_t n = R.cnt->n_mat[BIN];
     const uint32_t* q = R.q_mat[BIN];
     uint32_t* q_next = R.q_path[parity ^ 1];
@@ -1651,10 +1600,7 @@ __global__ void PB_SHADE_BOUNDS k_shade(RenderDev R, int parity) {
     // (instruction-cache misses) at 11 % issue-slot use.  Its CTA is the whole SM (PB_TEX_BLOCK threads at 128 registers) and its warps start every
     // path TOGETHER (barrier at the top of a trip; the queue is sorted by material, so they run the same programs): they fetch the same lines at
     // about the same time.  The trip count is CTA-uniform for the barrier.
-#ifndef PB_SHADE_SYNC
-#define PB_SHADE_SYNC 0  /* A/B: the same barrier in every bin's kernel (128-thread CTAs) */
-#endif
-    const bool lockstep = BIN == Q_TEX || PB_SHADE_SYNC;
+    const bool lockstep = BIN == Q_TEX;
     const uint32_t nround = lockstep ? ((n + blockDim.x - 1u) / blockDim.x) * blockDim.x : ((n + 31u) & ~31u);
     for (uint32_t i = blockIdx.x * blockDim.x + threadIdx.x; i < nround; i += gridDim.x * blockDim.x) {
         if (lockstep) __syncthreads();
@@ -1765,24 +1711,15 @@ struct ShadowJob {
     }
 };
 template <bool INST>
-__global__ void PB_TRACE_BOUNDS k_trace_shadow(RenderDev R) {
+__global__ void __launch_bounds__(PB_TRACE_BLOCK) k_trace_shadow(RenderDev R) {
     ShadowJob job{&R};
     trace_queue<true, INST, PB_SH_STACK>(R.scene, job, R.cnt->n_shadow, &R.cnt->fetch_shadow, TraceTune{PB_WF_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN});
 }
-#ifdef PB_TRACE_MINB_PLAIN_ANY  /* A/B knob (profiles/r02_ab_logs.md): the plain any-hit kernel alone */
-template <>
-__global__ void __launch_bounds__(PB_TRACE_BLOCK, PB_TRACE_MINB_PLAIN_ANY) k_trace_shadow<false>(RenderDev R) {
-    ShadowJob job{&R};
-    trace_queue<true, false, PB_SH_STACK>(R.scene, job, R.cnt->n_shadow, &R.cnt->fetch_shadow, TraceTune{PB_WF_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN});
-}
-#endif
-#if PB_TRACE_MINB_INST_ANY > 0
 template <>
 __global__ void __launch_bounds__(PB_TRACE_BLOCK, PB_TRACE_MINB_INST_ANY) k_trace_shadow<true>(RenderDev R) {
     ShadowJob job{&R};
     trace_queue<true, true, PB_SH_STACK>(R.scene, job, R.cnt->n_shadow, &R.cnt->fetch_shadow, TraceTune{PB_WF_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN});
 }
-#endif
 #endif  // PB_EXACT_TU
 
 // ---------------------------------------------------------------------------
@@ -1825,7 +1762,7 @@ struct MisJob {
     PB_D void store(uint32_t i, const TravRay& r) const { mis_resolve<INST>(*R, R->q_mis[i], r); }
 };
 template <bool INST>
-__global__ void PB_TRACE_BOUNDS k_trace_mis(RenderDev R) {
+__global__ void __launch_bounds__(PB_TRACE_BLOCK) k_trace_mis(RenderDev R) {
     MisJob<INST> job{&R};
     trace_queue<false, INST, PB_SH_STACK>(R.scene, job, R.cnt->n_mis, &R.cnt->fetch_mis, TraceTune{PB_WF_REFILL_BELOW, PB_FETCH_CHUNK, PB_INTERIOR_MIN});
 }
@@ -1838,7 +1775,7 @@ namespace pb {
 
 // Launchers of the kernels that live in the other translation unit (shade.o, see the top of this file)
 void launch_shade_kernels(const RenderDev& R, int parity, bool full, int grid_small, int grid_shade, cudaStream_t stream);
-void launch_rec_shade(const RenderDev& R, int parity, bool zt, bool full, int grid_shade, cudaStream_t stream);
+void launch_rec_shade(const RenderDev& R, int parity, bool zt, bool full, cudaStream_t stream);
 // ... and in mega.o
 void launch_zt_mega(const RenderDev& R, const RenderDev* rdev, uint32_t lanes, uint32_t nblk, cudaStream_t stream);
 void launch_vol_mega(const RenderDev& R, const RenderDev* rdev, unsigned long long total_items, int camera_medium, bool full, int grid, cudaStream_t stream);
@@ -1867,19 +1804,16 @@ void launch_shade_kernels(const RenderDev& R, int parity, bool full, int grid_sm
     if (full) launch_shade_family<true>(R, parity, grid_small, grid_shade, stream);
     else launch_shade_family<false>(R, parity, grid_small, grid_shade, stream);
 }
-void launch_rec_shade(const RenderDev& R, int parity, bool zt, bool full, int grid_shade, cudaStream_t stream) {
+void launch_rec_shade(const RenderDev& R, int parity, bool zt, bool full, cudaStream_t stream) {
+    static int g = 0;  // one CTA per SM
+    if (!g) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&g, cudaDevAttrMultiProcessorCount, dev); g = std::max(g, 1); }
     if (R.scene.material_ext) {
-        static int tex_grid = 0;  // one CTA per SM
-        if (!tex_grid) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&tex_grid, cudaDevAttrMultiProcessorCount, dev); tex_grid = std::max(tex_grid, 1); }
-        if (zt) k_rec_shade<true, true, true><<<tex_grid, PB_REC_TEX_BLOCK, 0, stream>>>(R, parity);
-        else k_rec_shade<true, false, true><<<tex_grid, PB_REC_TEX_BLOCK, 0, stream>>>(R, parity);
+        if (zt) k_rec_shade<true, true, true><<<g, PB_REC_BLOCK, 0, stream>>>(R, parity);
+        else k_rec_shade<true, false, true><<<g, PB_REC_BLOCK, 0, stream>>>(R, parity);
     } else {
-        static int rec_grid = 0;  // PB_REC_LOCKSTEP: one CTA per SM
-        if (!rec_grid) { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&rec_grid, cudaDevAttrMultiProcessorCount, dev); rec_grid = std::max(rec_grid, 1); }
-        const int g = PB_REC_LOCKSTEP ? rec_grid : grid_shade, b = PB_REC_LOCKSTEP ? PB_REC_TEX_BLOCK : 128;
-        if (zt) k_rec_shade<true, true, false><<<g, b, 0, stream>>>(R, parity);
-        else if (full) k_rec_shade<true, false, false><<<g, b, 0, stream>>>(R, parity);
-        else k_rec_shade<false, false, false><<<g, b, 0, stream>>>(R, parity);
+        if (zt) k_rec_shade<true, true, false><<<g, PB_REC_BLOCK, 0, stream>>>(R, parity);
+        else if (full) k_rec_shade<true, false, false><<<g, PB_REC_BLOCK, 0, stream>>>(R, parity);
+        else k_rec_shade<false, false, false><<<g, PB_REC_BLOCK, 0, stream>>>(R, parity);
     }
 }
 }  // namespace pb (shade.o ends here)
@@ -2305,12 +2239,6 @@ static __device__ __noinline__ ShadeOut vol_shade_medium(const RenderDev* Rp, ui
 template <int BIN, bool INST>
 static __device__ __noinline__ ShadeOut vol_shade(const RenderDev* Rp, uint32_t id, VolState* vs) { return shade_path<BIN, INST, false, true>(*Rp, id, vs); }
 
-#define PB_VOL_PHASED (PB_VOL_BLOCK > 64)
-#if PB_VOL_PHASED
-#define PB_VOL_SYNC() __syncthreads()
-#else
-#define PB_VOL_SYNC() ((void)0)
-#endif
 #define PB_VOL_SEGMENT_CAP 4096u   /* transmittance loops: boundaries crossed by one shadow / MIS ray before it is given up (hang guard) */
 #define PB_VOL_VERTEX_CAP 65536u   /* path loop: boundary crossings lower the bounce count, so max_depth alone does not bound it */
 template <bool INST>
@@ -2347,11 +2275,7 @@ __global__ void __launch_bounds__(PB_VOL_BLOCK) k_vol_mega(RenderDev R, const Re
         // ncu on the 64-thread form: issue slots 7 % busy, 52 of 57 stall cycles per instruction are `no_instruction` -- sixteen warps per SM each
         // somewhere else in 100s of KB of code miss the instruction cache all the time.  One 512-thread CTA per SM whose warps pass the phases of a
         // trip TOGETHER (barriers between trace / shade / shadow walk / MIS walk) keeps the SM inside one region of the code at a time.
-#if PB_VOL_PHASED
         if (!__syncthreads_or(have || !exhausted)) break;
-#else
-        if (!__any_sync(0xffffffffu, have || !exhausted)) break;
-#endif
         if (have) {
             if (vertices++ >= PB_VOL_VERTEX_CAP) alive = false;
         }
@@ -2368,7 +2292,7 @@ __global__ void __launch_bounds__(PB_VOL_BLOCK) k_vol_mega(RenderDev R, const Re
             bin = store_closest_hit(R, j, r);
             ms = vol_sample_medium(R, j, &vs, r.found, r.hit.t);
         }
-        PB_VOL_SYNC();
+        __syncthreads();
         ShadeOut o = {false, false, false, false, false};  // ms == 2: the path ends here (volpath.rs:114)
         if (have && alive) {
             if (ms == 2) {}
@@ -2385,7 +2309,7 @@ __global__ void __launch_bounds__(PB_VOL_BLOCK) k_vol_mega(RenderDev R, const Re
             }
             if (o.zero_rad) n_zero += 1;
         }
-        PB_VOL_SYNC();
+        __syncthreads();
         if (have && alive) {
             if (o.push_shadow) {  // VisibilityTester::tr, light.rs:125-150
                 float4 a = R.sh_ray[2 * j], b = R.sh_ray[2 * j + 1];
@@ -2417,7 +2341,7 @@ __global__ void __launch_bounds__(PB_VOL_BLOCK) k_vol_mega(RenderDev R, const Re
                 }
             }
         }
-        PB_VOL_SYNC();
+        __syncthreads();
         if (have && alive) {
             if (o.push_mis) {  // Scene::intersect_tr, scene.rs:68-87, then integrator.rs:218-232
                 float4 a = R.mis_ray[2 * j], b = R.mis_ray[2 * j + 1];
@@ -3148,8 +3072,6 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
     // shade kernels keep 5 CTAs of 128 threads resident per SM (96-104 registers): 10 per SM = two full waves (8 left a
     // 3-CTA tail wave: -1.5 % on S3, gpurun_out/ab4.log)
     int grid_shade = sm_count * 20, grid_small = sm_count * 4;  // shade: 10 -> 20 CTAs per SM: 35.4 -> 35.2 ms per 16-spp S3 step (gpurun_out/r2o_grid.log)
-    if (const char* e = getenv("PBRT_B200_GRID_SMALL")) grid_small = sm_count * std::max(1, atoi(e));  // A/B knobs (tools/ab_variants.sh)
-    if (const char* e = getenv("PBRT_B200_GRID_SHADE")) grid_shade = sm_count * std::max(1, atoi(e));
     if (zt) {  // tile-serial: at most one path per tile in flight -- a few CTAs cover the queues
         const int need = (int)((capacity + 127u) / 128u);
         grid_trace = std::min(grid_trace, need); grid_shade = std::min(grid_shade, need); grid_small = std::min(grid_small, need);
@@ -3284,7 +3206,6 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
             // tiles per warp, measured on B200 (gpurun_out/ab14.log): 625 tiles -> 2 lanes 7.1 M samples/s (1: 6.1, 4: 5.7); 8160 tiles ->
             // 8-16 lanes 11.2 M (1: 6.1, 32: 10.8); 32640 tiles -> 32 lanes 23.8 M (1: 6.5)
             uint32_t lanes = std::min<uint32_t>(32u, std::max<uint32_t>(1u, (n_tiles_sel + (uint32_t)sm_count * 4u - 1u) / ((uint32_t)sm_count * 4u)));
-            if (const char* e = getenv("PBRT_B200_ZT_LANES")) lanes = std::min<uint32_t>(32u, std::max<uint32_t>(1u, (uint32_t)atoi(e)));
             const uint32_t nblk = (n_tiles_sel + lanes * PB_ZT_WARPS - 1) / (lanes * PB_ZT_WARPS);
             launch_zt_mega(R, zt_rdev, lanes, nblk, stream);
             launches += 1;
@@ -3323,7 +3244,7 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
                     launches += 3;
                 }
                 if (R.rec.kind) {  // whitted / directlighting: one generic shade kernel, entry-indexed shadow and MIS rays
-                    launch_rec_shade(R, parity, zt, full, grid_shade, stream);
+                    launch_rec_shade(R, parity, zt, full, stream);
                     if (timing) mark();
                     if (inst) k_rec_shadow<true><<<grid_trace, PB_TRACE_BLOCK, 0, stream>>>(R);
                     else k_rec_shadow<false><<<grid_trace, PB_TRACE_BLOCK, 0, stream>>>(R);

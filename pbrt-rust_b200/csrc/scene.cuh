@@ -3,9 +3,6 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include "../../include/pbrt_b200.h"
-#ifndef PB_CQUAD
-#define PB_CQUAD 0 /* A/B build with compressed quad nodes: see trace.cuh */
-#endif
 
 namespace pb {
 
@@ -50,9 +47,6 @@ struct DevScene {
     //  q6 = {ref0, ref1, ref2, ref3}   q7 = {axis | axis_first << 2 | axis_second << 4, 0, 0, 0}
     // Used by rays without a zero direction component in scenes without instancing (trace.cuh: trav_run_quad).
     const float4* quads;
-#if PB_CQUAD
-    const float4* cquads;   // A/B: the same quad tree with 8-bit conservative child boxes, 64 B per node (trace.cuh: quad_step)
-#endif
     uint32_t n_fat;
     uint32_t root_ref;      // PB_REF_NONE when the scene is empty
     float root_box[6];      // LinearBVHNode[0].bounds = Scene.wb

@@ -12,43 +12,8 @@
 // parent is visited and only the t_max-dependent part of the reference's test
 // (`tmin < ray.t_max`) is re-evaluated when the entry is popped -- which is when the
 // reference would have tested that node.
+// Alternatives that were measured on B200 and lost are recorded in DESIGN.md §4 and profiles/ (r02_cquad.md, r02_trace_lanes.md).
 #pragma once
-#ifndef PB_PACKED_SLAB
-#define PB_PACKED_SLAB 1  /* FADD2/FMUL2 two-child slab test: +2-3% on B200 (tools/trace_ab3.py), bit-identical */
-#endif
-#ifndef PB_LEAN_SELECT
-#define PB_LEAN_SELECT 1  /* failed slab test folded into tmin = +inf, near child by (negmask >> axis): +3-4% on B200, bit-identical (gpurun_out/ab1.log) */
-#endif
-#ifndef PB_QUAD_NODES
-#define PB_QUAD_NODES 1  /* 128-byte quad nodes (four grandchildren per fetch) for rays without a zero direction component */
-#endif
-#ifndef PB_PREFETCH_FAR
-#define PB_PREFETCH_FAR 0
-#endif
-#ifndef PB_CQUAD
-#define PB_CQUAD 0  /* 1 (A/B, VERDICT n1): COMPRESSED quad nodes -- 64 B instead of 128: the four child boxes as 8-bit planes on a per-node power-of-two
-                       grid anchored at the node's lower corner (the CWBVH encoding of Ylitie et al. 2017, four wide), decoded in ray space with one
-                       FFMA per plane; the boxes are conservative (floor / ceil plus one quantum of slack), the visiting order is the reference's.
-                       Measured on B200 (profiles/r02_cquad.md): 8 M hit records bit-identical, camera batch -9 %, bounce batch -6 %, shadow batch -11 %,
-                       S3 frame -5.5 % (closest 14.4 -> 15.8 ms): the 77 MB of full-precision quad nodes already live in L2, the decode is serial work in
-                       front of the slab test, and the looser boxes are entered more often.  2: the same with the PRMT decode (see quad_step). */
-#endif
-#ifndef PB_LAZY_SHEAR
-#define PB_LAZY_SHEAR 0  /* 1: at instance boundaries the shear constants wait for the first triangle tested.  Measured on S4: +-0 (closest 230.7 -> 230.2 ms, shadow 69 -> 72 ms per 4-spp step) */
-#endif
-#ifndef PB_ANY_UNORDERED
-#define PB_ANY_UNORDERED 1  /* any-hit rays visit the four slots of a quad node in storage order: their answer does not depend on the order (t_max is
-                               constant), and the near / far selects are ~20 % of the node step.  B-shadow batch 4564 -> 4811 Mrays/s, occlusion bits identical */
-#endif
-#ifndef PB_COOP_TRAVERSAL
-#define PB_COOP_TRAVERSAL 0 /* 1: persistent ray queues walk the quad nodes warp-cooperatively, loop decisions are full-mask votes (trav_run_quad_coop).
-                               Measured on B200 (gpurun_out/r2d_ab.log): camera batch 4590 -> 4372 Mrays/s, S3 step 42.1 -> 43.2 ms, hits bit-identical:
-                               forcing the warp to converge removes the overlap of the leaf fetches of some lanes with the node fetches of others */
-#endif
-#ifndef PB_POSTPONE_LEAF
-#define PB_POSTPONE_LEAF 0  /* cooperative walk only: a lane that reaches a leaf parks it and keeps descending while the warp is still searching.
-                               Measured: camera batch 4202 Mrays/s, S3 step 47.8 ms (speculative descents under the stale t_max + 16 more registers) */
-#endif
 #include "scene.cuh"
 #include "vecmath.cuh"
 
@@ -232,24 +197,13 @@ PB_D bool slab_test(float nx, float ny, float nz, float fx, float fy, float fz, 
     return ok && (tmax > 0.0f);
 }
 
-// Same predicate and the same tmin for rays whose direction has no zero component: then no
+// Same predicate and the same tmin as slab_test for rays whose direction has no zero component: then no
 // product (b - o) * inv can be NaN, the reference's compare-and-assign chain equals max/min,
 // and its pairwise early-outs equal `tmin <= tmax` (the i == j pairs it skips can only fail
 // when that axis' far plane is behind the ray, which `tmax > 0` rejects anyway).
-PB_D bool slab_fast(float nx, float ny, float nz, float fx, float fy, float fz, f3 o, f3 inv, float* tmin_out) {
-    const float widen = 1.0f + 2.0f * gamma_n(3);
-    float tx0 = (nx - o.x) * inv.x, ty0 = (ny - o.y) * inv.y, tz0 = (nz - o.z) * inv.z;
-    float tx1 = (fx - o.x) * inv.x, ty1 = (fy - o.y) * inv.y, tz1 = (fz - o.z) * inv.z;
-    tx1 *= widen; ty1 *= widen; tz1 *= widen;
-    float tmin = fmaxf(fmaxf(tx0, ty0), tz0);
-    float tmax = fminf(fminf(tx1, ty1), tz1);
-    *tmin_out = tmin;
-    return (tmin <= tmax) && (tmax > 0.0f);
-}
-
-// Both children of a fat node at once with Blackwell's packed f32x2 pipe (FADD2 / FMUL2: two IEEE-rounded f32
-// results per issue slot).  Lane .x = child 0, .y = child 1.  Every product and difference is rounded exactly as in
-// slab_fast (sub -> mul -> mul can never contract), so the results are bit-identical.
+// Two boxes at once with Blackwell's packed f32x2 pipe (FADD2 / FMUL2: two IEEE-rounded f32 results per issue slot; +2-3 %
+// on B200 against the scalar form, tools/trace_ab3.py).  Lane .x = child 0, .y = child 1.  Every product and difference is
+// rounded exactly as in slab_test (sub -> mul -> mul can never contract), so the results are bit-identical.
 struct SlabPair { float tmin0, tmin1; bool ok0, ok1; };
 PB_D SlabPair slab_fast2(float2 nx, float2 ny, float2 nz, float2 fx, float2 fy, float2 fz, float2 nox, float2 noy, float2 noz, float2 ix, float2 iy, float2 iz) {
     const float w = 1.0f + 2.0f * gamma_n(3);
@@ -281,12 +235,9 @@ struct TravRay {
     f3 o, d, inv;
     float t_max, Sx, Sy, Sz;
     uint32_t cur;    // node / leaf reference being visited, or PB_DONE
-    uint32_t pend;   // quad walk with PB_POSTPONE_LEAF: the leaf reached but not yet tested, or PB_DONE
-    float cur_tmin;  // tmin of `cur`'s box as computed when it was stacked / chosen (re-validates a leaf reached under a stale t_max)
     int sp;
     int kx, ky, kz;
     bool ngx, ngy, ngz, found;
-    bool shear_ok;      // kz / Sx / Sy / Sz are valid for the current (o, d): see trav_set_ray<LAZY>
     uint32_t negmask;   // bit a set: the direction is negative along axis a
     bool nan_possible;  // a zero direction component: 0 * inf can appear in the slab test
     RayHit hit;
@@ -296,17 +247,11 @@ struct TravRay {
     bool inst_found;
     float world_t_max;
     f3 wo, wd;
-#if PB_PACKED_SLAB
     float2 nox, noy, noz, ivx, ivy, ivz;  // {-o, -o} and {1/d, 1/d} per axis for slab_fast2
-#endif
 };
 
-PB_D bool lane0_of_warp() { return (threadIdx.x & 31u) == 0u; }
-PB_D bool trav_done(const TravRay& r) { return r.cur == PB_DONE && r.pend == PB_DONE; }  // nothing left to visit, no parked leaf
+PB_D bool trav_done(const TravRay& r) { return r.cur == PB_DONE; }
 
-// root_ref / root_box: the accelerator to walk (the scene's aggregate or an instanced object's BVH); root_box == nullptr
-// for a one-primitive object, which the reference intersects directly (no accelerator, no bounds test)
-// everything the box and triangle tests derive from (o, d) alone
 // ray-constant part of the watertight test (triangle.rs:151-165)
 PB_D void trav_set_shear(TravRay& r) {
     const f3 d = r.d;
@@ -316,25 +261,17 @@ PB_D void trav_set_shear(TravRay& r) {
     r.ky = (r.kx + 1 == 3) ? 0 : r.kx + 1;
     const float dpx = comp(d, r.kx), dpy = comp(d, r.ky), dpz = comp(d, r.kz);
     r.Sx = -dpx / dpz; r.Sy = -dpy / dpz; r.Sz = 1.0f / dpz;
-    r.shear_ok = true;
 }
-// LAZY: leave the shear constants (three IEEE divisions) for the first triangle actually tested with this ray.  Used at
-// instance boundaries, where most rays that enter an object's box leave it again without reaching a leaf (S4: the six divisions
-// of the ray set-up at every instance entry and exit were 11 % of k_trace_closest<INST>'s warp instructions at 7 active lanes,
-// profiles/r02_s4_trace.md).
-template <bool LAZY = false>
+// everything the box and triangle tests derive from (o, d) alone
 PB_D void trav_set_ray(TravRay& r, f3 o, f3 d) {
     r.o = o; r.d = d;
     r.inv = f3(1.0f / d.x, 1.0f / d.y, 1.0f / d.z);
     r.ngx = r.inv.x < 0.0f; r.ngy = r.inv.y < 0.0f; r.ngz = r.inv.z < 0.0f;
     r.negmask = (r.ngx ? 1u : 0u) | (r.ngy ? 2u : 0u) | (r.ngz ? 4u : 0u);
     r.nan_possible = (d.x == 0.0f) || (d.y == 0.0f) || (d.z == 0.0f);
-#if PB_PACKED_SLAB
     r.nox = make_float2(-o.x, -o.x); r.noy = make_float2(-o.y, -o.y); r.noz = make_float2(-o.z, -o.z);
     r.ivx = make_float2(r.inv.x, r.inv.x); r.ivy = make_float2(r.inv.y, r.inv.y); r.ivz = make_float2(r.inv.z, r.inv.z);
-#endif
-    if (LAZY) r.shear_ok = false;
-    else trav_set_shear(r);
+    trav_set_shear(r);
 }
 // BVHAccel::intersect's first step: the root node's own bounds test (bvh.rs:724-727).  rb == nullptr: a one-primitive
 // object, which the reference intersects directly.
@@ -350,7 +287,6 @@ PB_D void trav_init_at(TravRay& r, f3 o, f3 d, float t_max, uint32_t root_ref, c
     r.t_max = t_max;
     r.hit.slot = PBRT_B200_NO_HIT; r.hit.t = t_max; r.hit.b0 = r.hit.b1 = r.hit.b2 = 0.0f; r.hit.inst = PBRT_B200_NO_HIT;
     r.found = false; r.sp = 0;
-    r.pend = PB_DONE; r.cur_tmin = -PB_INF;
     r.cur_inst = PBRT_B200_NO_HIT; r.inst_found = false;
     trav_set_ray(r, o, d);
     r.cur = trav_enter_root(r, root_ref, rb);
@@ -380,12 +316,8 @@ PB_D void xf_ray(const float* M, f3 o, f3 d, float t_max, f3* o_out, f3* d_out, 
 // per 16-spp step (closest 16.4 -> 16.1, shadow 8.1 -> 7.8 ms); on isolated 2 M-ray batches the same change LOSES 4-5 % (camera batch
 // 4603 -> 4390 Mrays/s: the carve-out shrinks the L1 that a small batch's nodes otherwise fit in).  So the wavefront kernels take the
 // hybrid stack and the batch API keeps the local one (trace_queue's SH parameter).
-#ifndef PB_SH_STACK
 #define PB_SH_STACK 16
-#endif
-#ifndef PB_TRACE_BLOCK
-#define PB_TRACE_BLOCK 128 /* threads per CTA of every persistent ray-queue kernel (util.cuh) */
-#endif
+#define PB_TRACE_BLOCK 128 /* threads per CTA of every persistent ray-queue kernel */
 struct LocalStack {
     uint2* loc;
     PB_D void put(int i, uint2 e) const { loc[i] = e; }
@@ -408,7 +340,7 @@ struct HybridStack {
         while ((r).sp > 0) {                                            \
             --(r).sp;                                                   \
             uint2 e__ = (stack).get((r).sp);                                \
-            if (__uint_as_float(e__.y) < (r).t_max) { (r).cur = e__.x; (r).cur_tmin = __uint_as_float(e__.y); break; } \
+            if (__uint_as_float(e__.y) < (r).t_max) { (r).cur = e__.x; break; } \
         }                                                               \
     } while (0)
 
@@ -418,47 +350,30 @@ template <bool ANY, typename STK> PB_D void quad_step(const DevScene& s, TravRay
 // lanes of the warp are still traversing, so that the caller can refill idle lanes.
 // TOP: walking the scene's aggregate (leaf slots may be TransformedPrimitives); false inside an instanced object, where
 // ObjectInstance cannot appear (api.rs:1674-1677): one level of instancing, one sentinel on the stack at most.
-template <bool ANY, bool EXACT_NAN, bool TOP, typename STK>
+// Boxes are tested with the literal reference chain (slab_test: exact for rays with a zero direction component); rays without
+// one take the quad step at TOP level, chosen per node visit because the ray changes at instance boundaries.
+template <bool ANY, bool TOP, typename STK>
 PB_D void trav_run_impl(const DevScene& s, TravRay& r, STK stack, int yield_below, int interior_min) {
     while (r.cur != PB_DONE) {
         // ---- interior nodes
         while (!(r.cur & PB_LEAF_BIT)) {
-#if PB_QUAD_NODES
-            // two-level walk: the ray changes at instance boundaries, so the NaN-free test is chosen per node visit
-            if (EXACT_NAN && TOP && !r.nan_possible) {
+            if (TOP && !r.nan_possible) {
                 quad_step<ANY>(s, r, stack);
                 if (interior_min > 0 && __popc(__activemask()) < interior_min) break;
                 continue;
             }
-#endif
             const float4* np = s.nodes + 4ull * r.cur;
             float4 q0 = __ldg(np), q1 = __ldg(np + 1), q2 = __ldg(np + 2), q3 = __ldg(np + 3);
             uint32_t ref0 = __float_as_uint(q3.x), ref1 = __float_as_uint(q3.y), axis = __float_as_uint(q3.z);
             float tmin0, tmin1;
-            bool ok0, ok1;
-            if (EXACT_NAN) {
-                ok0 = slab_test(r.ngx ? q0.w : q0.x, r.ngy ? q1.x : q0.y, r.ngz ? q1.y : q0.z, r.ngx ? q0.x : q0.w, r.ngy ? q0.y : q1.x,
-                                r.ngz ? q0.z : q1.y, r.o, r.inv, &tmin0);
-                ok1 = slab_test(r.ngx ? q2.y : q1.z, r.ngy ? q2.z : q1.w, r.ngz ? q2.w : q2.x, r.ngx ? q1.z : q2.y, r.ngy ? q1.w : q2.z,
-                                r.ngz ? q2.x : q2.w, r.o, r.inv, &tmin1);
-            } else {
-#if PB_PACKED_SLAB
-                SlabPair sp2 = slab_fast2(make_float2(r.ngx ? q0.w : q0.x, r.ngx ? q2.y : q1.z), make_float2(r.ngy ? q1.x : q0.y, r.ngy ? q2.z : q1.w),
-                                          make_float2(r.ngz ? q1.y : q0.z, r.ngz ? q2.w : q2.x), make_float2(r.ngx ? q0.x : q0.w, r.ngx ? q1.z : q2.y),
-                                          make_float2(r.ngy ? q0.y : q1.x, r.ngy ? q1.w : q2.z), make_float2(r.ngz ? q0.z : q1.y, r.ngz ? q2.x : q2.w),
-                                          r.nox, r.noy, r.noz, r.ivx, r.ivy, r.ivz);
-                ok0 = sp2.ok0; ok1 = sp2.ok1; tmin0 = sp2.tmin0; tmin1 = sp2.tmin1;
-#else
-                ok0 = slab_fast(r.ngx ? q0.w : q0.x, r.ngy ? q1.x : q0.y, r.ngz ? q1.y : q0.z, r.ngx ? q0.x : q0.w, r.ngy ? q0.y : q1.x,
-                                r.ngz ? q0.z : q1.y, r.o, r.inv, &tmin0);
-                ok1 = slab_fast(r.ngx ? q2.y : q1.z, r.ngy ? q2.z : q1.w, r.ngz ? q2.w : q2.x, r.ngx ? q1.z : q2.y, r.ngy ? q1.w : q2.z,
-                                r.ngz ? q2.x : q2.w, r.o, r.inv, &tmin1);
-#endif
-            }
+            const bool ok0 = slab_test(r.ngx ? q0.w : q0.x, r.ngy ? q1.x : q0.y, r.ngz ? q1.y : q0.z, r.ngx ? q0.x : q0.w, r.ngy ? q0.y : q1.x,
+                                       r.ngz ? q0.z : q1.y, r.o, r.inv, &tmin0);
+            const bool ok1 = slab_test(r.ngx ? q2.y : q1.z, r.ngy ? q2.z : q1.w, r.ngz ? q2.w : q2.x, r.ngx ? q1.z : q2.y, r.ngy ? q1.w : q2.z,
+                                       r.ngz ? q2.x : q2.w, r.o, r.inv, &tmin1);
             // near child = second child when the ray is negative along the split axis (bvh.rs:743-751)
-#if PB_LEAN_SELECT
             // a failed slab test becomes tmin = +inf: `tmin < t_max` is then false at the visit and at every later pop, which is
-            // all the reference ever asks of that box (an entry whose true tmin is +inf can never pass either)
+            // all the reference ever asks of that box (an entry whose true tmin is +inf can never pass either).  +3-4 % on B200
+            // against separate ok flags and a per-axis select of the near child, bit-identical.
             tmin0 = ok0 ? tmin0 : PB_INF; tmin1 = ok1 ? tmin1 : PB_INF;
             bool second_first = (r.negmask >> axis) & 1u;
             uint32_t nref = second_first ? ref1 : ref0, fref = second_first ? ref0 : ref1;
@@ -466,25 +381,9 @@ PB_D void trav_run_impl(const DevScene& s, TravRay& r, STK stack, int yield_belo
             bool nhit = ntmin < r.t_max;
             bool fhit = ftmin < r.t_max;
             bool fok = ANY ? fhit : (ftmin < PB_INF);
-#else
-            bool second_first = (axis == 0) ? r.ngx : ((axis == 1) ? r.ngy : r.ngz);
-            uint32_t nref = second_first ? ref1 : ref0, fref = second_first ? ref0 : ref1;
-            float ntmin = second_first ? tmin1 : tmin0, ftmin = second_first ? tmin0 : tmin1;
-            bool nok = second_first ? ok1 : ok0, fok = second_first ? ok0 : ok1;
-            bool nhit = nok && (ntmin < r.t_max);
-            // the far child's `tmin < t_max` is re-checked at pop time for closest-hit rays
-            // (t_max may have changed by then); for any-hit rays t_max is constant
-            bool fhit = fok && (ftmin < r.t_max);
-#endif
             if (nhit) {
                 if (ANY ? fhit : fok) {
                     stack.put(r.sp, make_uint2(fref, __float_as_uint(ftmin))); ++r.sp;
-#if PB_PREFETCH_FAR
-                    {
-                        const void* pf = (fref & PB_LEAF_BIT) ? (const void*)(s.tris + 3ull * (fref & ~PB_LEAF_BIT)) : (const void*)(s.nodes + 4ull * fref);
-                        asm volatile("prefetch.global.L2 [%0];" ::"l"(pf));
-                    }
-#endif
                 }
                 r.cur = nref;
             } else if (fhit) {
@@ -500,7 +399,7 @@ PB_D void trav_run_impl(const DevScene& s, TravRay& r, STK stack, int yield_belo
         if (TOP && r.cur == PB_INST_EXIT) {
             // back in world space: r.t_max = ray.t_max when the object was hit (primitive.rs:72), the world value otherwise
             if (!r.inst_found) r.t_max = r.world_t_max;
-            trav_set_ray<PB_LAZY_SHEAR != 0>(r, r.wo, r.wd);
+            trav_set_ray(r, r.wo, r.wd);
             r.cur_inst = PBRT_B200_NO_HIT; r.inst_found = false;
             PB_TRAV_POP(r, stack);
             continue;
@@ -530,7 +429,7 @@ PB_D void trav_run_impl(const DevScene& s, TravRay& r, STK stack, int yield_belo
                         float tm2;
                         xf_ray(in->world_to_prim, r.o, r.d, r.t_max, &o2, &d2, &tm2);
                         r.t_max = tm2;
-                        trav_set_ray<PB_LAZY_SHEAR != 0>(r, o2, d2);
+                        trav_set_ray(r, o2, d2);
                         r.cur = trav_enter_root(r, in->root_ref, (in->flags & PB_INST_HAS_BOX) ? in->root_box : nullptr);
                         entered = true;
                         break;
@@ -539,7 +438,6 @@ PB_D void trav_run_impl(const DevScene& s, TravRay& r, STK stack, int yield_belo
                     b0 = b1 = b2 = 0.0f;
                 } else {
                     f3 p0(v0.x, v0.y, v0.z), p1(v1.x, v1.y, v1.z), p2(v2.x, v2.y, v2.z);
-                    if (TOP && PB_LAZY_SHEAR && !r.shear_ok) trav_set_shear(r);
                     h = triangle_test<!ANY>(r.o, r.d, r.t_max, p0, p1, p2, r.kx, r.ky, r.kz, r.Sx, r.Sy, r.Sz, &t, &b0, &b1, &b2);
                     if (!ANY && h) {
                         float2 uv0, uv1, uv2;
@@ -576,62 +474,13 @@ PB_D void trav_run_impl(const DevScene& s, TravRay& r, STK stack, int yield_belo
 // every binary node.  The four slots are therefore walked in exactly that order (near group by the node's axis, near
 // slot inside each group by the child's axis), later ones are stacked behind earlier ones, and a stacked entry is
 // re-checked against the current t_max when popped, as in the binary walk.  Only for rays without zero direction
-// components (slab_fast's precondition; the others take the binary, NaN-exact walk).
+// components (slab_fast2's precondition; the others take the binary, NaN-exact walk).
 //
 // quad_slots: the four slots of quad node `node` in visiting order -- t[k] = the slot's tmin (+inf when its slab test fails), ref[k]
 // its reference.  The order depends on the ray only through `negmask` (trav_run_packet passes its warp's shared octant, which
 // makes ref[] warp-uniform).
 template <bool ANY>
 PB_D void quad_slots(const DevScene& s, const TravRay& r, uint32_t node, uint32_t negmask, float* t, uint32_t* ref) {
-#if PB_CQUAD
-    // {lower corner, ex | ey << 8 | ez << 16 | meta << 24}, {refs}, {lo.x[4], lo.y[4], lo.z[4], hi.x[4]}, {hi.y[4], hi.z[4], -, -}
-    const float4* np = s.cquads + 4ull * node;
-    const float4 hd = __ldg(np), q6 = __ldg(np + 1), qa = __ldg(np + 2), qb = __ldg(np + 3);
-    const uint32_t hb = __float_as_uint(hd.w);
-    // plane = corner + q * 2^e  ->  t = q * (2^e / d) + (corner - o) / d : one FFMA per plane (f32x2: two children per issue slot)
-    const float ax = __uint_as_float((hb & 0xffu) << 23) * r.ivx.x, ay = __uint_as_float(((hb >> 8) & 0xffu) << 23) * r.ivy.x, az = __uint_as_float(((hb >> 16) & 0xffu) << 23) * r.ivz.x;
-#if PB_CQUAD == 2
-    // decode variant: a byte becomes the float 2^23 + q with one PRMT (I2F.U8 runs on the quarter-rate conversion pipe) and the 2^23 is folded into the
-    // constant term.  Faster than I2F (profiles/r02_cquad.md) but the fold's rounding (up to half a quantum) is not covered at the corner planes, which
-    // have no slack below q = 0: 27-388 of 2 M hit records differ.  Kept for the timing only.
-    const float bx = __fmaf_rn(-8388608.0f, ax, (hd.x + r.nox.x) * r.ivx.x), by = __fmaf_rn(-8388608.0f, ay, (hd.y + r.noy.x) * r.ivy.x),
-                bz = __fmaf_rn(-8388608.0f, az, (hd.z + r.noz.x) * r.ivz.x);
-#else
-    const float bx = (hd.x + r.nox.x) * r.ivx.x, by = (hd.y + r.noy.x) * r.ivy.x, bz = (hd.z + r.noz.x) * r.ivz.x;
-#endif
-    const float2 Ax = make_float2(ax, ax), Ay = make_float2(ay, ay), Az = make_float2(az, az), Bx = make_float2(bx, bx), By = make_float2(by, by), Bz = make_float2(bz, bz);
-    const uint32_t lox = __float_as_uint(qa.x), loy = __float_as_uint(qa.y), loz = __float_as_uint(qa.z), hix = __float_as_uint(qa.w), hiy = __float_as_uint(qb.x), hiz = __float_as_uint(qb.y);
-    const uint32_t wnx = r.ngx ? hix : lox, wny = r.ngy ? hiy : loy, wnz = r.ngz ? hiz : loz, wfx = r.ngx ? lox : hix, wfy = r.ngy ? loy : hiy, wfz = r.ngz ? loz : hiz;
-#if PB_CQUAD == 2
-#define PB_Q01(w) make_float2(__uint_as_float(__byte_perm((w), 0x4B000000u, 0x7540)), __uint_as_float(__byte_perm((w), 0x4B000000u, 0x7541)))
-#define PB_Q23(w) make_float2(__uint_as_float(__byte_perm((w), 0x4B000000u, 0x7542)), __uint_as_float(__byte_perm((w), 0x4B000000u, 0x7543)))
-#else
-#define PB_Q01(w) make_float2((float)((w) & 0xffu), (float)(((w) >> 8) & 0xffu))
-#define PB_Q23(w) make_float2((float)(((w) >> 16) & 0xffu), (float)((w) >> 24))
-#endif
-    const float wdn = 1.0f + 2.0f * gamma_n(3);
-    const float2 widen = make_float2(wdn, wdn);
-    SlabPair pa, pb;
-    {
-        const float2 tx0 = __ffma2_rn(PB_Q01(wnx), Ax, Bx), ty0 = __ffma2_rn(PB_Q01(wny), Ay, By), tz0 = __ffma2_rn(PB_Q01(wnz), Az, Bz);
-        const float2 tx1 = __fmul2_rn(__ffma2_rn(PB_Q01(wfx), Ax, Bx), widen), ty1 = __fmul2_rn(__ffma2_rn(PB_Q01(wfy), Ay, By), widen), tz1 = __fmul2_rn(__ffma2_rn(PB_Q01(wfz), Az, Bz), widen);
-        pa.tmin0 = fmaxf(fmaxf(tx0.x, ty0.x), tz0.x); pa.tmin1 = fmaxf(fmaxf(tx0.y, ty0.y), tz0.y);
-        const float m0 = fminf(fminf(tx1.x, ty1.x), tz1.x), m1 = fminf(fminf(tx1.y, ty1.y), tz1.y);
-        pa.ok0 = (pa.tmin0 <= m0) && (m0 > 0.0f) && __float_as_uint(q6.x) != PB_REF_NONE;
-        pa.ok1 = (pa.tmin1 <= m1) && (m1 > 0.0f) && __float_as_uint(q6.y) != PB_REF_NONE;
-    }
-    {
-        const float2 tx0 = __ffma2_rn(PB_Q23(wnx), Ax, Bx), ty0 = __ffma2_rn(PB_Q23(wny), Ay, By), tz0 = __ffma2_rn(PB_Q23(wnz), Az, Bz);
-        const float2 tx1 = __fmul2_rn(__ffma2_rn(PB_Q23(wfx), Ax, Bx), widen), ty1 = __fmul2_rn(__ffma2_rn(PB_Q23(wfy), Ay, By), widen), tz1 = __fmul2_rn(__ffma2_rn(PB_Q23(wfz), Az, Bz), widen);
-        pb.tmin0 = fmaxf(fmaxf(tx0.x, ty0.x), tz0.x); pb.tmin1 = fmaxf(fmaxf(tx0.y, ty0.y), tz0.y);
-        const float m0 = fminf(fminf(tx1.x, ty1.x), tz1.x), m1 = fminf(fminf(tx1.y, ty1.y), tz1.y);
-        pb.ok0 = (pb.tmin0 <= m0) && (m0 > 0.0f) && __float_as_uint(q6.z) != PB_REF_NONE;
-        pb.ok1 = (pb.tmin1 <= m1) && (m1 > 0.0f) && __float_as_uint(q6.w) != PB_REF_NONE;
-    }
-#undef PB_Q01
-#undef PB_Q23
-    const float4 q7 = make_float4(__uint_as_float(hb >> 24), 0.0f, 0.0f, 0.0f);
-#else
     const float4* np = s.quads + 8ull * node;
     const float4 a0 = __ldg(np), a1 = __ldg(np + 1), a2 = __ldg(np + 2), b0 = __ldg(np + 3), b1 = __ldg(np + 4), b2 = __ldg(np + 5), q6 = __ldg(np + 6), q7 = __ldg(np + 7);
     SlabPair pa = slab_fast2(r.ngx ? make_float2(a1.z, a1.w) : make_float2(a0.x, a0.y), r.ngy ? make_float2(a2.x, a2.y) : make_float2(a0.z, a0.w),
@@ -642,7 +491,6 @@ PB_D void quad_slots(const DevScene& s, const TravRay& r, uint32_t node, uint32_
                              r.ngz ? make_float2(b2.z, b2.w) : make_float2(b1.x, b1.y), r.ngx ? make_float2(b0.x, b0.y) : make_float2(b1.z, b1.w),
                              r.ngy ? make_float2(b0.z, b0.w) : make_float2(b2.x, b2.y), r.ngz ? make_float2(b1.x, b1.y) : make_float2(b2.z, b2.w),
                              r.nox, r.noy, r.noz, r.ivx, r.ivy, r.ivz);
-#endif
     const float tA0 = pa.ok0 ? pa.tmin0 : PB_INF, tA1 = pa.ok1 ? pa.tmin1 : PB_INF, tB0 = pb.ok0 ? pb.tmin0 : PB_INF, tB1 = pb.ok1 ? pb.tmin1 : PB_INF;
     const uint32_t meta = __float_as_uint(q7.x);
     const bool g = (negmask >> (meta & 3u)) & 1u, sA = (negmask >> ((meta >> 2) & 3u)) & 1u, sB = (negmask >> ((meta >> 4) & 3u)) & 1u;
@@ -650,15 +498,11 @@ PB_D void quad_slots(const DevScene& s, const TravRay& r, uint32_t node, uint32_
     const float tAn = sA ? tA1 : tA0, tAf = sA ? tA0 : tA1, tBn = sB ? tB1 : tB0, tBf = sB ? tB0 : tB1;
     const uint32_t rAn = __float_as_uint(sA ? q6.y : q6.x), rAf = __float_as_uint(sA ? q6.x : q6.y);
     const uint32_t rBn = __float_as_uint(sB ? q6.w : q6.z), rBf = __float_as_uint(sB ? q6.z : q6.w);
-#if PB_ANY_UNORDERED
-    // A/B: an any-hit ray's answer does not depend on the visiting order (t_max never changes): slots in storage order, no selects
+    // an any-hit ray's answer does not depend on the visiting order (t_max never changes): slots in storage order, no selects (the
+    // near / far selects are ~20 % of the node step: shadow batch 4564 -> 4811 Mrays/s on B200, occlusion bits identical)
     const float t0 = ANY ? tA0 : (g ? tBn : tAn), t1 = ANY ? tA1 : (g ? tBf : tAf), t2 = ANY ? tB0 : (g ? tAn : tBn), t3 = ANY ? tB1 : (g ? tAf : tBf);
     const uint32_t r0 = ANY ? __float_as_uint(q6.x) : (g ? rBn : rAn), r1 = ANY ? __float_as_uint(q6.y) : (g ? rBf : rAf),
                    r2 = ANY ? __float_as_uint(q6.z) : (g ? rAn : rBn), r3 = ANY ? __float_as_uint(q6.w) : (g ? rAf : rBf);
-#else
-    const float t0 = g ? tBn : tAn, t1 = g ? tBf : tAf, t2 = g ? tAn : tBn, t3 = g ? tAf : tBf;
-    const uint32_t r0 = g ? rBn : rAn, r1 = g ? rBf : rAf, r2 = g ? rAn : rBn, r3 = g ? rAf : rBf;
-#endif
     t[0] = t0; t[1] = t1; t[2] = t2; t[3] = t3;
     ref[0] = r0; ref[1] = r1; ref[2] = r2; ref[3] = r3;
 }
@@ -671,25 +515,13 @@ PB_D void quad_step(const DevScene& s, TravRay& r, STK stack) {
     const uint32_t r0 = ref[0], r1 = ref[1], r2 = ref[2], r3 = ref[3];
     // the first slot that passes is visited now; the others wait on the stack, nearest on top
     uint32_t nref = PB_DONE; float ntm = 0.0f;
-#if PB_PREFETCH_FAR
-    uint32_t top = PB_DONE;  // the entry left on top of the stack by this step: the next thing visited after the subtree entered now
-#define PB_QPUSH() do { stack.put(r.sp, make_uint2(nref, __float_as_uint(ntm))); ++r.sp; top = nref; } while (0)
-#else
 #define PB_QPUSH() do { stack.put(r.sp, make_uint2(nref, __float_as_uint(ntm))); ++r.sp; } while (0)
-#endif
     if (t3 < r.t_max) { nref = r3; ntm = t3; }
     if (t2 < r.t_max) { if (nref != PB_DONE) PB_QPUSH(); nref = r2; ntm = t2; }
     if (t1 < r.t_max) { if (nref != PB_DONE) PB_QPUSH(); nref = r1; ntm = t1; }
     if (t0 < r.t_max) { if (nref != PB_DONE) PB_QPUSH(); nref = r0; ntm = t0; }
 #undef PB_QPUSH
-#if PB_PREFETCH_FAR
-    // A/B: request it into L1 now (ncu: 38 % of the node / leaf fetches miss L1)
-    if (top != PB_DONE) {
-        const void* pf = (top & PB_LEAF_BIT) ? (const void*)(s.tris + 3ull * (top & ~PB_LEAF_BIT)) : (const void*)(s.quads + 8ull * top);
-        asm volatile("prefetch.global.L1 [%0];" ::"l"(pf));
-    }
-#endif
-    if (nref != PB_DONE) { r.cur = nref; r.cur_tmin = ntm; }
+    if (nref != PB_DONE) r.cur = nref;
     else PB_TRAV_POP(r, stack);
 }
 // Every primitive of leaf `first_slot`, in order (bvh.rs:730-736).  Returns true when an any-hit ray is finished.
@@ -740,62 +572,6 @@ PB_D void trav_run_quad(const DevScene& s, TravRay& r, STK stack, int yield_belo
             PB_TRAV_POP(r, stack);
         }
         if (yield_below > 0 && __popc(__activemask()) < yield_below) break;
-    }
-}
-
-// WARP-COOPERATIVE form for the persistent ray queues: ALL 32 lanes of the warp call it together (lanes without a ray ride
-// along, predicated off) and every loop decision is a full-mask vote, so the two hot bodies really run converged.  ncu on the
-// per-lane form (whose loop exits the compiler does not reconverge: lanes that reach a leaf run ahead into the triangle
-// test while the others keep descending) measured 5 of 32 lanes active in the triangle test and 18 in the node step
-// (profiles/r02_trace_lanes.md).
-//
-// PB_POSTPONE_LEAF: a lane that reaches a leaf parks it in `pend` and goes on with the traversal (pop, descend) while
-// the rest of the warp is still searching, instead of idling; the leaf body runs when fewer than `interior_min` lanes are
-// still looking for their first leaf.  Exactness (same leaves, same order, same t_max at every test as the reference):
-// t_max changes only in the leaf body and a lane parks at most one leaf, so a parked leaf was validated against the t_max
-// the reference would have used.  What the lane does while a leaf is parked happens under a STALE (larger) t_max, which
-// can only admit more boxes: every stack entry is re-checked against the current t_max when popped (as before), and a
-// leaf reached meanwhile waits in `cur` until the parked leaf has been tested, then is re-checked with its own box tmin
-// (`cur_tmin`); tmin is monotone down the tree (see the quad-node note above), so a leaf that passes implies that every
-// box on the way to it passes.  Leaves are found in depth-first order and tested first-in first-out: ties break as in
-// the reference.
-template <bool ANY, typename STK>
-PB_D void trav_run_quad_coop(const DevScene& s, TravRay& r, STK stack, int yield_below, int interior_min) {
-    const unsigned FULL = 0xffffffffu;
-    const int min_searching = interior_min > 0 ? interior_min : 1;
-    for (;;) {
-        // ---- node steps until fewer than `min_searching` lanes are still looking for a leaf
-        for (;;) {
-            if (!(r.cur & PB_LEAF_BIT)) quad_step<ANY>(s, r, stack);
-#if PB_POSTPONE_LEAF
-            if (r.pend == PB_DONE && (r.cur & PB_LEAF_BIT) && r.cur != PB_DONE) { r.pend = r.cur; PB_TRAV_POP(r, stack); }
-            const bool searching = r.pend == PB_DONE && !(r.cur & PB_LEAF_BIT);
-#else
-            const bool searching = !(r.cur & PB_LEAF_BIT);
-#endif
-            if (__popc(__ballot_sync(FULL, searching)) < min_searching) break;
-        }
-        // ---- leaf bodies, converged
-#if PB_POSTPONE_LEAF
-        if (r.pend != PB_DONE) {
-            const uint32_t leaf = r.pend & ~PB_LEAF_BIT;
-            r.pend = PB_DONE;
-            if (quad_leaf_run<ANY>(s, r, leaf)) { r.cur = PB_DONE; r.sp = 0; }
-        }
-        __syncwarp(FULL);
-        // a second leaf reached under the stale t_max: re-validate, park it, move on
-        if ((r.cur & PB_LEAF_BIT) && r.cur != PB_DONE) {
-            if (ANY || r.cur_tmin < r.t_max) r.pend = r.cur;
-            PB_TRAV_POP(r, stack);
-        }
-#else
-        if ((r.cur & PB_LEAF_BIT) && r.cur != PB_DONE) {
-            if (quad_leaf_run<ANY>(s, r, r.cur & ~PB_LEAF_BIT)) { r.cur = PB_DONE; r.sp = 0; }
-            else PB_TRAV_POP(r, stack);
-        }
-#endif
-        const int alive = __popc(__ballot_sync(FULL, !trav_done(r)));
-        if (alive == 0 || alive < yield_below) break;
     }
 }
 
@@ -860,14 +636,10 @@ PB_D void trav_run_packet(const DevScene& s, TravRay& r, STK stack, uint32_t neg
 // contain no trace of the instance path (measured on S3: the mere presence of the out-of-line call in the leaf loop costs 20%).
 template <bool ANY, bool INST, typename STK>
 PB_D void trav_run(const DevScene& s, TravRay& r, STK stack, int yield_below, int interior_min = 0) {
-    // with instances the ray changes along the way, so the NaN-free slab shortcut cannot be chosen once per ray: INST
-    // kernels always evaluate the literal reference chain
-    if (INST || r.nan_possible) trav_run_impl<ANY, true, INST>(s, r, stack, yield_below, interior_min);
-#if PB_QUAD_NODES
+    // with instances the ray changes along the way, so the quad walk cannot be chosen once per ray: INST kernels choose it per
+    // node visit (trav_run_impl)
+    if (INST || r.nan_possible) trav_run_impl<ANY, INST>(s, r, stack, yield_below, interior_min);
     else trav_run_quad<ANY>(s, r, stack, yield_below, interior_min);
-#else
-    else trav_run_impl<ANY, false, INST>(s, r, stack, yield_below, interior_min);
-#endif
 }
 
 // Closest-hit (ANY=false) or any-hit (ANY=true) traversal of one ray, run to completion.
@@ -983,18 +755,13 @@ PB_D bool traverse_ifif(const DevScene& s, f3 o, f3 d, float t_max, RayHit* hit)
 // Refill latency.  A warp's refill is one atomicAdd on a single global counter -- ~1 M of them per 33 M-ray launch, one every ~5 ns
 // against the ~4 ns the L2 slice needs per same-address atomic (profiles/r02_ncu_regen.md) -- whose round trip the whole warp waits
 // for.  Two ways around it were tried and BOTH measured slower on B200 (hits bit-identical; gpurun_out/r2j_ab.log, r2k_ab.log):
-//   * PB_FETCH_AHEAD = 1: lane 0 reserves the NEXT chunk while the current one is traversed (one chunk of look-ahead per warp):
+//   * lane 0 reserves the NEXT chunk while the current one is traversed (one chunk of look-ahead per warp):
 //     S3 step 35.8 -> 37.2 ms, camera batch 4424 -> 4244 Mrays/s;
 //   * reserving 4 / 8 chunks per global atomic and parking the extra ones in shared memory for the sibling warps: 35.8 -> 37.6 / 40.1 ms.
 // Both widen the band of the ray queue that is in flight at any moment; the queue is in path order (neighbouring pixels, then
 // neighbouring hit points), and the traversal's cache hit rates live off that locality more than they suffer from the refill wait.
-#ifndef PB_FETCH_AHEAD
-#define PB_FETCH_AHEAD 0
-#endif
 #define PB_REFILL_BELOW 24
-#ifndef PB_INTERIOR_MIN
 #define PB_INTERIOR_MIN 16
-#endif
 struct TraceTune { int refill_below; int chunk; int interior_min; };
 // The shared levels of the hybrid stack: one array per kernel, which trace_queue and trace_queue_packet both use.
 template <int SH>
@@ -1007,13 +774,9 @@ PB_D void trace_queue(const DevScene& s, Job& job, uint32_t n, uint32_t* fetch_c
     uint2 stack_mem[PB_STACK_SIZE(INST)];
     HybridStack<SH, PB_TRACE_BLOCK> stack{trace_stack_shared<SH>(), stack_mem};  // SH == 0: every level in the local array
     TravRay r;
-    r.cur = PB_DONE; r.pend = PB_DONE; r.sp = 0; r.found = false;
+    r.cur = PB_DONE; r.sp = 0; r.found = false;
     uint32_t ray_idx = 0xffffffffu;
     uint32_t pool_next = 0, pool_end = 0;  // warp-uniform
-#if PB_FETCH_AHEAD
-    uint32_t ahead = 0;
-    if (lane0_of_warp()) ahead = atomicAdd(fetch_counter, (uint32_t)tune.chunk);
-#endif
     bool exhausted = false;                // warp-uniform
     const unsigned lane = threadIdx.x & 31u;
     const unsigned lt_mask = (1u << lane) - 1u;
@@ -1025,13 +788,7 @@ PB_D void trace_queue(const DevScene& s, Job& job, uint32_t n, uint32_t* fetch_c
         while (need && !exhausted) {
             if (pool_next == pool_end) {
                 uint32_t b = 0;
-#if PB_FETCH_AHEAD
-                // the chunk reserved when the previous one was taken (its atomic has had a whole chunk's traversal to complete);
-                // the reservation for the refill after this one goes out now
-                if (lane == 0) { b = ahead; ahead = atomicAdd(fetch_counter, (uint32_t)tune.chunk); }
-#else
                 if (lane == 0) b = atomicAdd(fetch_counter, (uint32_t)tune.chunk);
-#endif
                 b = __shfl_sync(0xffffffffu, b, 0);
                 if (b >= n) { exhausted = true; break; }
                 pool_next = b; pool_end = min(b + (uint32_t)tune.chunk, n);
@@ -1044,22 +801,13 @@ PB_D void trace_queue(const DevScene& s, Job& job, uint32_t n, uint32_t* fetch_c
                 ray_idx = pool_next + rank;
                 f3 o, d; float t_max = 0.0f;
                 if (job.load(ray_idx, &o, &d, &t_max)) trav_init(s, r, o, d, t_max);
-                else { r.cur = PB_DONE; r.pend = PB_DONE; r.sp = 0; r.found = false; r.hit.slot = PBRT_B200_NO_HIT; r.hit.t = t_max; r.hit.inst = PBRT_B200_NO_HIT; }
+                else { r.cur = PB_DONE; r.sp = 0; r.found = false; r.hit.slot = PBRT_B200_NO_HIT; r.hit.t = t_max; r.hit.inst = PBRT_B200_NO_HIT; }
             }
             unsigned took = __ballot_sync(0xffffffffu, take);
             pool_next += __popc(took);
             need &= ~took;
         }
         if (__all_sync(0xffffffffu, ray_idx == 0xffffffffu)) break;
-#if PB_QUAD_NODES && PB_COOP_TRAVERSAL
-        if (!INST) {
-            // rays with a zero direction component take the NaN-exact binary walk (rare): run them to completion first
-            if (r.nan_possible && !trav_done(r)) trav_run_impl<ANY, true, false>(s, r, stack, 0, 0);
-            __syncwarp();
-            trav_run_quad_coop<ANY>(s, r, stack, exhausted ? 0 : tune.refill_below, tune.interior_min);
-            continue;
-        }
-#endif
         trav_run<ANY, INST>(s, r, stack, exhausted ? 0 : tune.refill_below, tune.interior_min);
     }
 }
@@ -1080,7 +828,7 @@ PB_D void trace_queue_packet(const DevScene& s, Job& job, uint32_t n, uint32_t* 
         if (b >= n) break;
         const uint32_t idx = b + lane;
         TravRay r;
-        r.cur = PB_DONE; r.pend = PB_DONE; r.sp = 0; r.found = false;
+        r.cur = PB_DONE; r.sp = 0; r.found = false;
         r.hit.slot = PBRT_B200_NO_HIT; r.hit.inst = PBRT_B200_NO_HIT;
         f3 o, d; float t_max = 0.0f;
         if (idx < n) {

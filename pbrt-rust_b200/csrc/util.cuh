@@ -1,11 +1,9 @@
-// CUDA error plumbing and launch constants.
+// CUDA error plumbing.
 #pragma once
 #include <cuda_runtime.h>
 #include <string>
 #include "error.h"
 #include "../../include/pbrt_b200.h"
-
-#define PB_TRACE_BLOCK 128
 
 #define PB_CUDA_TRY(call)                                                                              \
     do {                                                                                               \

@@ -137,7 +137,7 @@ def load_library():
     if _lib is not None:
         return _lib
     import os
-    path = Path(os.environ.get("PBRT_B200_LIB", LIB_PATH))  # A/B builds (csrc/Makefile `variant`); still a CUDA library, never a fallback
+    path = Path(os.environ.get("PBRT_B200_LIB", LIB_PATH))  # a second build for before/after comparisons (csrc/Makefile NAME=...); still a CUDA library, never a fallback
     if not path.exists():
         raise B200Error(f"{path} is missing: run `python -c 'import __graft_entry__ as g; g.build()'` (no CPU fallback exists)")
     lib = C.CDLL(str(path))

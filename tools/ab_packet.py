@@ -3,7 +3,7 @@
 The arms are values of PBRT_B200_PACKET_TRAVERSAL, which pbrt_b200_render reads per call ("off": 0, the per-lane walk
 everywhere; "on": unset, the default).  Arms alternate step by step and render the same sample ranges; each arm's film and
 ray counts are checked against the first arm's.  Prints per-arm medians of the step time and of the traversal kernels' times.
-PBRT_B200_LIB selects another build of the library (csrc/Makefile: make variant)."""
+PBRT_B200_LIB selects another build of the library (csrc/Makefile: make NAME=<name>)."""
 import importlib
 import os
 import statistics

@@ -1,7 +1,7 @@
 """A/B timing of the batch traversal kernels on the three ray populations of a path-traced frame of S3:
 tile-ordered camera rays, bounce-1 rays (cosine-ish hemisphere about the hit normal) and shadow rays toward the
-area light.  Run once per library build:  PBRT_B200_LIB=pbrt-rust_b200/libpbrt_b200_<variant>.so python tools/trace_ab3.py
-Prints Mrays/s per (tune, batch) and a CRC of the results so variants can be compared for bit-equality."""
+area light.  Run once per library build (csrc/Makefile: make NAME=<name>):  PBRT_B200_LIB=pbrt-rust_b200/libpbrt_b200_<name>.so python tools/trace_ab3.py
+Prints Mrays/s per (tune, batch) and a CRC of the results so builds can be compared for bit-equality."""
 import importlib, sys, ctypes as C, math, os, zlib
 sys.path.insert(0, '.')
 import numpy as np
