@@ -63,7 +63,7 @@ PB_D f3 normalize(f3 a) { return vdiv(a, len(a)); }
 PB_D f3 vabs(f3 a) { return f3(fabsf(a.x), fabsf(a.y), fabsf(a.z)); }
 // geometry/vector.rs:339-353: f64 products, then narrowed
 #ifdef PB_TU_SHADE
-// shade.o (tolerance-parity shading, see render.cu): plain f32
+// shade.cu (tolerance-parity shading, see there): plain f32
 PB_D f3 cross(f3 a, f3 b) { return f3(a.y * b.z - a.z * b.y, a.z * b.x - a.x * b.z, a.x * b.y - a.y * b.x); }
 #else
 PB_D f3 cross(f3 a, f3 b) {

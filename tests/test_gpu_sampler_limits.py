@@ -1,6 +1,6 @@
 """The path integrator at the limits of its sampler and film bookkeeping, against the CPU oracle.
 
-Sobol' sample values reach the shade kernels three ways (render.cu, PathSampler<false>): rows of the per-pixel and
+Sobol' sample values reach the shade kernels three ways (path.cuh, PathSampler<false>): rows of the per-pixel and
 per-sample tables, the pre-pass k_sample_block (Halton, and Sobol' dimensions the tables do not hold), and, past the
 1024 dimensions of the generator matrices, the constant 0.5 (the oracle reads 0.5 there too; the reference panics).  The
 three give bit-identical values, so renders in every mode take the same paths.  PBRT_B200_NO_SOBOL_TABLES turns the
@@ -226,7 +226,7 @@ def test_deep_paths_across_halton_prime_table(pkg, oracle, gpu_lib, maxdepth):
     _check_oracle(oracle, integ, got, st, want, ost, ray_tol=DEEP_RAY_TOL)
 
 
-VOL_VERTEX_CAP = 65536  # PB_VOL_VERTEX_CAP, render.cu
+VOL_VERTEX_CAP = 65536  # PB_VOL_VERTEX_CAP, mega.cu
 
 
 @gpu

@@ -1,4 +1,4 @@
-"""VolPathIntegrator on the GPU (k_vol_mega, csrc/render.cu) against the CPU oracle (oracle/oracle_volpath.hpp).
+"""VolPathIntegrator on the GPU (k_vol_mega, csrc/mega.cu) against the CPU oracle (oracle/oracle_volpath.hpp).
 
 Same gate as the surface path integrator: image relMSE <= 1e-3 (north_star), equal camera-ray counts, ray counts within
 0.3 % (a path whose medium / Russian-roulette decision sits on a rounding boundary -- expf / logf differ by an ulp
