@@ -288,13 +288,26 @@ typedef struct pbrt_b200_integrator {
     uint32_t reserved;
 } pbrt_b200_integrator;
 
-/* = HomogeneousMedium (src/media/homogeneous.rs:10-27) with its HenyeyGreenstein phase function (medium.rs:172-200). 32 B. */
+/* = HomogeneousMedium (src/media/homogeneous.rs:10-27) or GridDensityMedium (src/media/grid.rs) with its HenyeyGreenstein phase
+ * function (medium.rs:172-200). 32 B. */
 typedef struct pbrt_b200_medium {
     float sigma_a[3];
     float sigma_s[3];                /* sigma_t = sigma_a + sigma_s is formed on use, as HomogeneousMedium::new does */
     float g;
-    float pad;
+    uint32_t grid;                   /* 0: HomogeneousMedium; k > 0: GridDensityMedium whose density grid is grids[k - 1] of
+                                      * pbrt_b200_scene_create_with_grids.  A grid medium uses sigma_t = (sigma_a + sigma_s)[0]. */
 } pbrt_b200_medium;
+
+/* The density field of a GridDensityMedium (src/media/grid.rs).  medium_to_world maps the unit box [0,1]^3 of the grid onto
+ * the world (CTM at MakeNamedMedium x Translate(p0) x Scale(p1 - p0)); world_to_medium is its inverse as the Transform
+ * carries it.  Both row-major.  density[(z * ny + y) * nx + x] is the value at voxel (x, y, z), nx * ny * nz floats,
+ * finite and >= 0.  152 B. */
+typedef struct pbrt_b200_density_grid {
+    float medium_to_world[16];
+    float world_to_medium[16];
+    uint32_t nx, ny, nz, pad;
+    const float *density;
+} pbrt_b200_density_grid;
 
 /* = MediumInterface of a GeometricPrimitive (src/core/medium.rs:131-160, primitive.rs:105-150): indices into `media`, -1 = none.
  * A row whose two sides differ is a medium transition; other rows inherit the medium of the ray that hits them.        */
@@ -369,6 +382,11 @@ int pbrt_b200_device_count(void);
 
 /* Scene::new (src/core/scene.rs:32-52) + upload.  `device` = CUDA ordinal.     */
 int pbrt_b200_scene_create(const pbrt_b200_scene_desc *desc, int device, pbrt_b200_scene **out);
+/* The same with the density grids the media rows refer to (pbrt_b200_medium.grid).  scene_create(d, dev, out) is
+ * scene_create_with_grids(d, NULL, 0, dev, out).  The densities are copied; a grid is checked before anything reaches the
+ * device (index range, non-null density, nx * ny * nz > 0 without overflow, finite non-negative densities, finite matrices). */
+int pbrt_b200_scene_create_with_grids(const pbrt_b200_scene_desc *desc, const pbrt_b200_density_grid *grids, uint64_t n_grids, int device,
+                                      pbrt_b200_scene **out);
 void pbrt_b200_scene_destroy(pbrt_b200_scene *scene);
 /* Scene.wb (scene.rs:27): root bounds, 6 floats. */
 int pbrt_b200_scene_world_bound(const pbrt_b200_scene *scene, float *bounds6);

@@ -7,9 +7,11 @@ functions.  `WorldEnd` does what `API::world_end` does up to the call of `Integr
 (api.rs:1715-1747): it flattens the scene into the tables of `pbrt_b200_scene_desc`, builds the BVH through
 `pbrt_b200_bvh_build` and assembles film / camera / sampler / integrator; the result is a `RenderJob` whose
 `render(device)` runs the CUDA path.  Anything the device path does not implement (other integrators, shapes and
-materials, alpha cut-outs, grid media, image-mapped infinite lights, non-perspective cameras) raises `B200Error` naming the
+materials, alpha cut-outs, media presets, image-mapped infinite lights, non-perspective cameras) raises `B200Error` naming the
 feature: there is no CPU fallback and no silent substitution.  Textures (every class of src/textures/, image maps through
-MIPMap pyramids), bump maps, `uber` / `substrate` and homogeneous media are on the device path since round 2.
+MIPMap pyramids), bump maps, `uber` / `substrate`, homogeneous media and heterogeneous (grid density) media are on the device
+path.  One deliberate deviation there: a heterogeneous medium without `density` values, or with
+a count other than nx * ny * nz, raises `B200Error` where the reference logs an error and creates no medium.
 
 Reference behaviours kept on purpose (each cited where it is implemented): `Camera` registers the camera space
 under the name "name", not "camera" (api.rs:1210); `ActiveTransform` never restricts which transform a
@@ -220,9 +222,7 @@ class API:
         if not ty:
             self._error('No parameter string "type" found in MakeNamedMedium')
             return
-        if ty == "heterogeneous":
-            raise B200Error('Medium "heterogeneous" (GridDensityMedium) is outside the hot path (homogeneous)')
-        if ty != "homogeneous":
+        if ty not in ("homogeneous", "heterogeneous"):
             warnings.warn(f'Medium "{ty}" unknown.')
             return
         preset = params.find_one_string("preset", "")
@@ -232,8 +232,14 @@ class API:
         g = float(params.find_one_float("g", 0.0))
         siga = params.find_one_spectrum("sigma_a", np.array([0.0011, 0.0024, 0.014], f32))
         sigs = params.find_one_spectrum("sigma_s", np.array([2.55, 3.21, 3.77], f32))
+        grid = {}
+        if ty == "heterogeneous":  # GridDensityMedium; missing or miscounted density raises B200Error (SceneBuilder.make_named_medium)
+            grid = {"density": params.find_float("density"), "nx": params.find_one_int("nx", 1), "ny": params.find_one_int("ny", 1),
+                    "nz": params.find_one_int("nz", 1), "p0": params.find_one_point3f("p0", (0.0, 0.0, 0.0)),
+                    "p1": params.find_one_point3f("p1", (1.0, 1.0, 1.0))}
         params.report_unused()
-        self.builder.make_named_medium(name, type=ty, sigma_a=siga, sigma_s=sigs, g=g, scale=scale)
+        self.builder.ctm = self.ctm  # a grid's medium_to_world starts from the CTM at MakeNamedMedium (api.rs make_medium)
+        self.builder.make_named_medium(name, type=ty, sigma_a=siga, sigma_s=sigs, g=g, scale=scale, **grid)
 
     def _medium_names(self):  # create_medium_interface, api.rs:382-403: an undefined name is logged and stands for no medium
         out = []

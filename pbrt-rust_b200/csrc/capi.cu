@@ -1,5 +1,6 @@
 // C-ABI entry points: scene upload and the batch intersect API (include/pbrt_b200.h).
 #include <cuda_runtime.h>
+#include <cmath>
 #include <cstdio>
 #include <cstring>
 #include <string>
@@ -291,6 +292,45 @@ int validate_mipmaps(const pbrt_b200_scene_desc* d) {
         uint32_t big = m.width > m.height ? m.width : m.height, levels = 1;
         while (big > 1) { big >>= 1; levels += 1; }
         if (m.n_levels != levels) return fail(PBRT_B200_ERR_INVALID, "scene_create: mipmap n_levels must be 1 + log2(max(width, height))");
+    }
+    return PBRT_B200_OK;
+}
+
+// Grid shapes are checked before anything is staged (the uploader sizes its copies from them); the values are scanned on the
+// table-check thread (validate_grid_values).
+int validate_grid_shapes(const pbrt_b200_density_grid* grids, uint64_t n_grids) {
+    if (n_grids && !grids) return fail(PBRT_B200_ERR_INVALID, "scene_create: grids is null");
+    if (n_grids > 0x7fffffffull) return fail(PBRT_B200_ERR_INVALID, "scene_create: too many density grids");
+    for (uint64_t i = 0; i < n_grids; ++i) {
+        const pbrt_b200_density_grid& g = grids[i];
+        if (!g.density) return fail(PBRT_B200_ERR_INVALID, "scene_create: density grid without density values");
+        const uint64_t nxy = (uint64_t)g.nx * g.ny;  // < 2^64: both factors are 32-bit
+        if (g.nx == 0 || g.ny == 0 || g.nz == 0 || nxy > (1ull << 40) / g.nz)
+            return fail(PBRT_B200_ERR_INVALID, "scene_create: density grid nx * ny * nz must be positive and at most 2^40");
+        for (int k = 0; k < 16; ++k)
+            if (!std::isfinite(g.medium_to_world[k]) || !std::isfinite(g.world_to_medium[k]))
+                return fail(PBRT_B200_ERR_INVALID, "scene_create: density grid matrices must be finite");
+    }
+    return PBRT_B200_OK;
+}
+
+// Every medium row's grid index, then every density (finite, >= 0) and each grid's maximum (GridDensityMedium::new).
+int validate_grid_values(const pbrt_b200_scene_desc* d, const pbrt_b200_density_grid* grids, uint64_t n_grids, std::vector<float>* max_density) {
+    for (uint64_t i = 0; i < d->n_media; ++i)
+        if (d->media[i].grid > n_grids) return fail(PBRT_B200_ERR_INVALID, "scene_create: medium grid index out of range");
+    max_density->assign(n_grids, 0.0f);
+    for (uint64_t i = 0; i < n_grids; ++i) {
+        const pbrt_b200_density_grid& g = grids[i];
+        const uint64_t n = (uint64_t)g.nx * g.ny * g.nz;
+        float m = 0.0f;
+        bool ok = true;
+        for (uint64_t k = 0; k < n; ++k) {
+            const float v = g.density[k];
+            ok = ok && v >= 0.0f && v < INFINITY;  // false for NaN
+            m = v > m ? v : m;
+        }
+        if (!ok) return fail(PBRT_B200_ERR_INVALID, "scene_create: densities must be finite and non-negative");
+        (*max_density)[i] = m;
     }
     return PBRT_B200_OK;
 }
@@ -597,6 +637,11 @@ extern "C" void pbrt_b200_scene_destroy(pbrt_b200_scene* sc) {
 }
 
 extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device, pbrt_b200_scene** out) {
+    return pbrt_b200_scene_create_with_grids(d, nullptr, 0, device, out);
+}
+
+extern "C" int pbrt_b200_scene_create_with_grids(const pbrt_b200_scene_desc* d, const pbrt_b200_density_grid* grids, uint64_t n_grids, int device,
+                                                 pbrt_b200_scene** out) {
     if (!d || !out) return fail(PBRT_B200_ERR_INVALID, "scene_create: null argument");
     *out = nullptr;
     const bool prof = getenv("PBRT_B200_PROFILE") != nullptr;
@@ -611,6 +656,8 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
     if (d->n_prims && !d->prims) return fail(PBRT_B200_ERR_INVALID, "scene_create: prims is null");
     if (d->n_nodes && !d->nodes) return fail(PBRT_B200_ERR_INVALID, "scene_create: nodes is null");
     if (int rcm = validate_mipmaps(d)) return rcm;
+    if (int rcg = validate_grid_shapes(grids, n_grids)) return rcg;
+    std::vector<float> max_density;
     // The table checks (index ranges, BVH structure and depth: ~10 ms for 10^6 primitives) run on two worker threads
     // while this thread stages the tables into HBM; nothing on the device dereferences an index before they have passed.
     int rc = PBRT_B200_OK, rc_v = PBRT_B200_OK, rc_n = PBRT_B200_OK;
@@ -621,7 +668,10 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
         f();
         if (prof) fprintf(stderr, "[pbrt_b200] scene_create   (%s: %.3f ms)\n", what, std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now() - a).count());
     };
-    std::thread th_v([&] { timed("table checks", [&] { rc_v = validate(d); }); if (rc_v) err_v = pbrt_b200::last_error_cstr(); });
+    std::thread th_v([&] {
+        timed("table checks", [&] { rc_v = validate(d); if (!rc_v) rc_v = validate_grid_values(d, grids, n_grids, &max_density); });
+        if (rc_v) err_v = pbrt_b200::last_error_cstr();
+    });
     std::vector<uint32_t> obj_fat_base;
     std::thread th_n([&] { timed("BVH checks", [&] { rc_n = check_nodes(d, &n_interior, &root_ref, &obj_fat_base); }); if (rc_n) err_n = pbrt_b200::last_error_cstr(); });
     struct Joiner { std::thread &a, &b; ~Joiner() { if (a.joinable()) a.join(); if (b.joinable()) b.join(); } } joiner{th_v, th_n};
@@ -659,6 +709,9 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
     add(sizeof(pbrt_b200_texnode) * d->n_textures); add(sizeof(pbrt_b200_mipmap) * d->n_mipmaps);
     add(d->material_ext ? sizeof(pbrt_b200_material_ext) * d->n_materials : 0);
     for (uint64_t i = 0; i < d->n_mipmaps; ++i) add(4 * mip_floats(d->mipmaps[i]));
+    auto grid_floats = [](const pbrt_b200_density_grid& g) { return (size_t)g.nx * g.ny * g.nz; };
+    add(sizeof(DevGrid) * n_grids);
+    for (uint64_t i = 0; i < n_grids; ++i) add(4 * grid_floats(grids[i]));
     const size_t resident = need;
     add(sizeof(pbrt_b200_bvh_node) * nn); add(4ull * nn); add(4ull * nb);
     need += 4096;
@@ -731,9 +784,27 @@ extern "C" int pbrt_b200_scene_create(const pbrt_b200_scene_desc* d, int device,
     }
     up(mips.data(), sizeof(pbrt_b200_mipmap) * mips.size(), &ds.mipmaps);
     if (err == cudaSuccess && !mips.empty()) err = cudaStreamSynchronize(stream);  // `mips` is a local: its copy must have been read
+    std::vector<DevGrid> dev_grids(n_grids);
+    for (uint64_t i = 0; i < n_grids; ++i) {
+        DevGrid& g = dev_grids[i];
+        std::memcpy(g.world_to_medium, grids[i].world_to_medium, sizeof g.world_to_medium);
+        g.nx = grids[i].nx; g.ny = grids[i].ny; g.nz = grids[i].nz;
+        up(grids[i].density, 4 * grid_floats(grids[i]), &g.density);
+    }
     lap("h2d staged");
     if ((rc = join_checks())) { pbrt_b200_scene_destroy(sc); return rc; }
     lap("checks joined");
+    bool grid_media = false;  // render.cu runs the grid kernel only for scenes whose media use a grid
+    for (uint64_t i = 0; i < d->n_media; ++i) grid_media = grid_media || d->media[i].grid > 0;
+    if (grid_media) {  // the maxima come from the table-check thread
+        for (uint64_t i = 0; i < n_grids; ++i) {
+            dev_grids[i].max_density = max_density[i];
+            dev_grids[i].inv_max_density = 1.0f / max_density[i];  // GridDensityMedium::new; +inf for an all-zero grid (vacuum: never used)
+        }
+        up(dev_grids.data(), sizeof(DevGrid) * n_grids, &sc->grids);
+        sc->n_grids = (uint32_t)n_grids;
+        if (err == cudaSuccess) err = cudaStreamSynchronize(stream);  // `dev_grids` is a local
+    }
     // read on this thread only now: until the table checks have passed, `lights` may be null with a non-zero count
     ds.n_sphere_lights = 0;
     for (uint64_t i = 0; i < d->n_lights; ++i)

@@ -1089,7 +1089,11 @@ struct ShadeOut { bool push_next, push_shadow, push_mis, push_dead, zero_rad; };
 // VOL: VolPathIntegrator::li's surface branch (volpath.rs:134-189) -- the same vertex, except that the light is sampled whatever the
 // BSDF's lobes are (no num_components test), rays carry a medium (`vs`), and a material-less surface LOWERS the bounce count
 // (`bounces -= 1; continue` skips the loop's increment; at 0 the usize wraps and the path ends at its next depth test).
-template <int BIN, bool INST, bool ZT, bool VOL = false>
+// PART (volpath with grid media, where estimate_direct's transmittance loops draw from the sampler and so must run between the two
+// halves of the vertex): 0 = the whole vertex; 1 = up to and including the light sample -- a vertex that goes on returns neither
+// push_next nor push_dead, its continuation is pending; 2 = the continuation (next direction, roulette), which recomputes the
+// interaction and the BSDF from the hit record still in the slot.
+template <int BIN, bool INST, bool ZT, bool VOL = false, int PART = 0>
 PB_D ShadeOut shade_path(const RenderDev& R, uint32_t id, VolState* vs = nullptr) {
     constexpr int KM = BinKinds<BIN>::KM;
     (void)KM;
@@ -1122,7 +1126,7 @@ PB_D ShadeOut shade_path(const RenderDev& R, uint32_t id, VolState* vs = nullptr
         else si = surface_at_hit<INST>(R.scene, hinst, h.x, ro, rd, __uint_as_float(h.y), __uint_as_float(h.z), __uint_as_float(h.w), R.hit_b2[id], &fl);
         const pbrt_b200_prim pr = R.scene.prims[h.x];
         // SurfaceInteraction::le, interaction.rs:344-349 + AreaLight::l, diffuse.rs:68-75
-        if ((bounces == 0 || specular_bounce) && pr.area_light >= 0) {
+        if constexpr (PART != 2) if ((bounces == 0 || specular_bounce) && pr.area_light >= 0) {
             const pbrt_b200_light& al = R.scene.lights[pr.area_light];
             if (al.two_sided || dot(si.n, -rd) > 0.0f) L = L + rgb3(al.L) * beta;
         }
@@ -1155,7 +1159,7 @@ PB_D ShadeOut shade_path(const RenderDev& R, uint32_t id, VolState* vs = nullptr
                 smp.begin(R, id);
                 const int NONSPEC = BX_ALL & ~BX_SPECULAR;
                 // ---- uniform_sample_onelight + estimate_direct, integrator.rs:81-237
-                if ((VOL || bsdf_count(bsdf, NONSPEC) > 0) && R.n_lights > 0) {
+                if constexpr (PART != 2) if ((VOL || bsdf_count(bsdf, NONSPEC) > 0) && R.n_lights > 0) {
                     float u1 = smp.get_1d();
                     // light_distrib.lookup(isect.p), path.rs:132
                     const float* ld_cdf = R.ld_cdf; const float* ld_func = R.ld_func; float ld_func_int = R.ld_func_int;
@@ -1218,6 +1222,11 @@ PB_D ShadeOut shade_path(const RenderDev& R, uint32_t id, VolState* vs = nullptr
                         }
                     }
                     zero_rad = zero;
+                }
+                if constexpr (PART == 1) {  // the continuation is pending (phase 5 of k_vol_mega<.., true>)
+                    R.L_eta[id] = make_float4(L.r, L.g, L.b, etascale);
+                    smp.end(R, id);
+                    return ShadeOut{false, push_shadow, push_mis, false, zero_rad};
                 }
                 // ---- sample the BSDF for the next direction, path.rs:147-174
                 f3 wo = -rd, wi(0.f, 0.f, 0.f);
@@ -1344,7 +1353,8 @@ void launch_shade_kernels(const RenderDev& R, int parity, bool full, int grid_sm
 void launch_rec_shade(const RenderDev& R, int parity, bool zt, bool full, cudaStream_t stream);
 // ... and in mega.cu
 void launch_zt_mega(const RenderDev& R, const RenderDev* rdev, uint32_t lanes, uint32_t nblk, cudaStream_t stream);
-void launch_vol_mega(const RenderDev& R, const RenderDev* rdev, unsigned long long total_items, int camera_medium, bool full, int grid, cudaStream_t stream);
-int vol_mega_blocks_per_sm(bool full);
+void launch_vol_mega(const RenderDev& R, const RenderDev* rdev, unsigned long long total_items, int camera_medium, bool full, const DevGrid* grids, int grid,
+                     cudaStream_t stream);
+int vol_mega_blocks_per_sm(bool full, bool grids);
 
 }  // namespace pb

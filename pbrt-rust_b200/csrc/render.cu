@@ -1060,7 +1060,7 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
     if (vol) {
         int smc = 148, per_sm = 1;
         cudaDeviceGetAttribute(&smc, cudaDevAttrMultiProcessorCount, sc->device);
-        per_sm = vol_mega_blocks_per_sm(sc->dev.n_instances || sc->dev.n_sphere_lights || sc->dev.material_ext);
+        per_sm = vol_mega_blocks_per_sm(sc->dev.n_instances || sc->dev.n_sphere_lights || sc->dev.material_ext, sc->grids != nullptr);
         const unsigned long long want = (total_items + (unsigned long long)PB_VOL_BLOCK - 1ull) / (unsigned long long)PB_VOL_BLOCK;
         vol_grid = (int)std::max<unsigned long long>(1ull, std::min<unsigned long long>((unsigned long long)smc * (unsigned long long)std::max(per_sm, 1), want));
         capacity = ((uint32_t)vol_grid * (uint32_t)PB_VOL_BLOCK + 255u) & ~255u;
@@ -1292,7 +1292,8 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
             if (!rdev) return fail(PBRT_B200_ERR_CUDA, "render: out of device memory");
             ZtRelease rdev_release{rdev, rdev_bytes};
             PB_CUDA_TRY(cudaMemcpyAsync(rdev, &R, sizeof(RenderDev), cudaMemcpyHostToDevice, stream));
-            launch_vol_mega(R, rdev, total_items, rd->integrator.camera_medium, sc->dev.n_instances || sc->dev.n_sphere_lights || sc->dev.material_ext, vol_grid, stream);
+            launch_vol_mega(R, rdev, total_items, rd->integrator.camera_medium, sc->dev.n_instances || sc->dev.n_sphere_lights || sc->dev.material_ext, sc->grids,
+                            vol_grid, stream);
             launches += 1;
             PB_CUDA_TRY(cudaGetLastError());
             PB_CUDA_TRY(cudaStreamSynchronize(stream));  // rdev is released at the end of this block

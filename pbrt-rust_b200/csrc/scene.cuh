@@ -30,6 +30,16 @@ struct DevInstance {
     float root_box[6];     // object BVH root bounds; a one-primitive object has no accelerator (api.rs:1691) and no box test
 };
 
+// GridDensityMedium (src/media/grid.rs) as the volpath grid kernel reads it: pbrt_b200_density_grid with the density moved to the
+// device and max_density found by scene_create (0 for an all-zero grid, which sample and tr treat as vacuum).
+struct DevGrid {
+    float world_to_medium[16];
+    uint32_t nx, ny, nz;
+    float max_density;
+    float inv_max_density;  // 1 / max_density
+    const float* density;   // density[(z * ny + y) * nx + x]
+};
+
 struct DevScene {
     // Fat BVH2: per INTERIOR node of the reference's LinearBVHNode array, the exact f32
     // boxes of both children (48 B) + child refs + split axis = 64 B = 4 x float4:
@@ -109,4 +119,6 @@ struct pbrt_b200_scene {
     void* light_distrib = nullptr;  // owned by render.cu
     uint32_t* fetch_counter = nullptr;  // device counter of the persistent ray queue (batch API)
     int trace_grid = 0;
+    const pb::DevGrid* grids = nullptr;  // density grids of the media rows with grid > 0 (device table of n_grids rows)
+    uint32_t n_grids = 0;
 };

@@ -15,6 +15,7 @@ from __future__ import annotations
 import ctypes as C
 import math
 import os
+import warnings
 from pathlib import Path
 
 import numpy as np
@@ -50,7 +51,10 @@ assert NODE_DTYPE.itemsize == 32 and PRIM_DTYPE.itemsize == 24 and SPHERE_DTYPE.
 assert MATERIAL_DTYPE.itemsize == 48 and LIGHT_DTYPE.itemsize == 136 and RAY_DTYPE.itemsize == 32 and HIT_DTYPE.itemsize == 16
 
 SHAPE_TRIANGLE, SHAPE_SPHERE, SHAPE_INSTANCE = 0, 1, 2
-MEDIUM_DTYPE = np.dtype([("sigma_a", "<f4", 3), ("sigma_s", "<f4", 3), ("g", "<f4"), ("pad", "<f4")])                      # pbrt_b200_medium
+MEDIUM_DTYPE = np.dtype([("sigma_a", "<f4", 3), ("sigma_s", "<f4", 3), ("g", "<f4"), ("grid", "<u4")])                     # pbrt_b200_medium
+DENSITY_GRID_DTYPE = np.dtype([("medium_to_world", "<f4", 16), ("world_to_medium", "<f4", 16), ("nx", "<u4"), ("ny", "<u4"), ("nz", "<u4"),
+                               ("pad", "<u4"), ("density", "<u8")])                                                              # pbrt_b200_density_grid
+assert DENSITY_GRID_DTYPE.itemsize == 152
 MEDIUM_INTERFACE_DTYPE = np.dtype([("inside", "<i4"), ("outside", "<i4")])                                                   # pbrt_b200_medium_interface
 OBJECT_DTYPE = np.dtype([("node_offset", "<u8"), ("n_nodes", "<u8"), ("prim_offset", "<u8"), ("n_prims", "<u8")])
 INSTANCE_DTYPE = np.dtype([("prim_to_world", "<f4", 16), ("world_to_prim", "<f4", 16), ("object", "<u4"), ("pad", "<u4", 3)])
@@ -117,7 +121,7 @@ RENDER_KEEP_ON_DEVICE = 1
 RENDER_LAZY_SPATIAL = 2
 RENDER_OVERWRITE = 4
 
-EXPORTS = ["pbrt_b200_last_error", "pbrt_b200_abi_version", "pbrt_b200_device_count", "pbrt_b200_bvh_build", "pbrt_b200_scene_create",
+EXPORTS = ["pbrt_b200_last_error", "pbrt_b200_abi_version", "pbrt_b200_device_count", "pbrt_b200_bvh_build", "pbrt_b200_scene_create", "pbrt_b200_scene_create_with_grids",
            "pbrt_b200_scene_destroy", "pbrt_b200_scene_world_bound", "pbrt_b200_intersect", "pbrt_b200_intersect_p", "pbrt_b200_intersect_dev",
            "pbrt_b200_intersect_p_dev", "pbrt_b200_render", "pbrt_b200_film_resolve", "pbrt_b200_light_distribution_lookup", "pbrt_b200_release_cached_memory", "pbrt_b200_tile_positions",
            "pbrt_b200_work_counter_open", "pbrt_b200_work_counter_fetch_add", "pbrt_b200_work_counter_fetch_max", "pbrt_b200_work_counter_load", "pbrt_b200_work_counter_store",
@@ -144,6 +148,7 @@ def load_library():
     lib.pbrt_b200_last_error.restype = C.c_char_p
     lib.pbrt_b200_bvh_build.argtypes = [C.c_void_p, C.c_uint64, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)]
     lib.pbrt_b200_scene_create.argtypes = [C.POINTER(SceneDesc), C.c_int, C.POINTER(C.c_void_p)]
+    lib.pbrt_b200_scene_create_with_grids.argtypes = [C.POINTER(SceneDesc), C.c_void_p, C.c_uint64, C.c_int, C.POINTER(C.c_void_p)]
     lib.pbrt_b200_scene_destroy.argtypes = [C.c_void_p]
     lib.pbrt_b200_scene_destroy.restype = None
     lib.pbrt_b200_scene_world_bound.argtypes = [C.c_void_p, C.c_void_p]
@@ -411,6 +416,17 @@ def bvh_build(prim_bounds, max_prims=4, split_method="sah"):
     return nodes[: nn.value].copy(), ordered[:n].copy()
 
 
+class DensityGrid:
+    """The density field of a GridDensityMedium (grid.rs): density[(z * ny + y) * nx + x] over the unit box that medium_to_world
+    (4x4, row-major) maps into the world; world_to_medium is its inverse as the Transform carries it."""
+
+    def __init__(self, density, nx, ny, nz, medium_to_world, world_to_medium):
+        self.density = np.ascontiguousarray(density, f32).reshape(-1)
+        self.nx, self.ny, self.nz = int(nx), int(ny), int(nz)
+        self.medium_to_world = np.ascontiguousarray(medium_to_world, f32).reshape(4, 4)
+        self.world_to_medium = np.ascontiguousarray(world_to_medium, f32).reshape(4, 4)
+
+
 class FlatScene:
     """The arrays behind `pbrt_b200_scene_desc` (owned here; the library copies them)."""
 
@@ -428,7 +444,8 @@ class FlatScene:
         self.objects = np.zeros(0, OBJECT_DTYPE)
         self.instances = np.zeros(0, INSTANCE_DTYPE)
         self.n_top_nodes = self.n_top_prims = 0  # 0 = all of nodes / prims (no object instancing)
-        self.media = np.zeros(0, MEDIUM_DTYPE)       # HomogeneousMedium rows (volpath)
+        self.media = np.zeros(0, MEDIUM_DTYPE)       # HomogeneousMedium / GridDensityMedium rows (volpath)
+        self.grids = []                              # DensityGrid of each media row with grid = k > 0 (grids[k - 1])
         self.prim_media = None                       # MediumInterface per `prims` row, or None
         self.textures = np.zeros(0, T.TEXNODE_DTYPE)  # postfix texture programs (ABI v5)
         self.mipmaps = np.zeros(0, T.MIPMAP_DTYPE)    # rows point into the MipMap objects kept in mipmap_objects
@@ -464,6 +481,14 @@ class FlatScene:
                 raise B200Error("FlatScene.prim_media must have one row per primitive row")
             d.prim_media = _ptr(self.prim_media)
         return d
+
+    def grid_table(self):
+        """pbrt_b200_density_grid rows of `grids`; their density pointers stay valid while this FlatScene lives."""
+        t = np.zeros(len(self.grids), DENSITY_GRID_DTYPE)
+        for k, g in enumerate(self.grids):
+            t[k]["medium_to_world"], t[k]["world_to_medium"] = g.medium_to_world.reshape(-1), g.world_to_medium.reshape(-1)
+            t[k]["nx"], t[k]["ny"], t[k]["nz"], t[k]["density"] = g.nx, g.ny, g.nz, g.density.ctypes.data
+        return t
 
     @property
     def world_bound(self):
@@ -520,6 +545,7 @@ class SceneBuilder:
         self._objects, self._instances, self._cur_object = {}, [], None
         # participating media (api.rs:1211-1258): named media are global (RenderOptions), the current interface is graphics state
         self._media, self._media_index = [], {}
+        self._grids = []                # DensityGrid of each heterogeneous medium, in creation order
         self._medium_names = ("", "")   # (inside, outside) of GraphicsState
         self._pmedia = []               # one [n,2] int32 block per entry of self._prims: MediumInterface of each primitive row
         self.log = []  # every directive in call order (scenefile.py turns it back into a .pbrt file)
@@ -566,19 +592,42 @@ class SceneBuilder:
         self.ctm, self._material, self._area_light, self.reverse_orientation, self._medium_names = self._stack.pop()
 
     # --- participating media (api.rs:706-760,1211-1258) -----------------------
-    def make_named_medium(self, name, type="homogeneous", sigma_a=(0.0011, 0.0024, 0.014), sigma_s=(2.55, 3.21, 3.77), g=0.0, scale=1.0, preset=""):
-        """MakeNamedMedium (api.rs:1211-1241 -> make_medium :706-760): defaults as there; sigma_a / sigma_s are multiplied by `scale`."""
-        self.log.append(("MakeNamedMedium", name, {"type": type, "sigma_a": tuple(np.asarray(sigma_a, f32).reshape(-1).tolist()) if not np.isscalar(sigma_a) else sigma_a,
-                                                   "sigma_s": tuple(np.asarray(sigma_s, f32).reshape(-1).tolist()) if not np.isscalar(sigma_s) else sigma_s,
-                                                   "g": g, "scale": scale}))
-        if type != "homogeneous":
-            raise B200Error(f'Medium "{type}" is outside the hot path (homogeneous)')
+    def make_named_medium(self, name, type="homogeneous", sigma_a=(0.0011, 0.0024, 0.014), sigma_s=(2.55, 3.21, 3.77), g=0.0, scale=1.0, preset="",
+                          density=None, nx=1, ny=1, nz=1, p0=(0.0, 0.0, 0.0), p1=(1.0, 1.0, 1.0)):
+        """MakeNamedMedium (api.rs:1211-1241 -> make_medium :706-760): defaults as there; sigma_a / sigma_s are multiplied by `scale`.
+
+        type="heterogeneous" is a GridDensityMedium (grid.rs): `density` holds nx * ny * nz values, x fastest, over the box p0..p1
+        of the current transformation.  Its sigma_t is (sigma_a + sigma_s)[0], the first channel only, as the reference's
+        constructor takes it; a sigma_t that is not the same in every channel draws a warning.  Where the reference logs an error and
+        creates no medium -- `density` missing, or not nx * ny * nz values -- this raises B200Error, so that a smoke scene whose data
+        failed to load is refused instead of rendered as vacuum."""
+        kw = {"type": type, "sigma_a": tuple(np.asarray(sigma_a, f32).reshape(-1).tolist()) if not np.isscalar(sigma_a) else sigma_a,
+              "sigma_s": tuple(np.asarray(sigma_s, f32).reshape(-1).tolist()) if not np.isscalar(sigma_s) else sigma_s, "g": g, "scale": scale}
+        if type == "heterogeneous":
+            kw.update({"nx": int(nx), "ny": int(ny), "nz": int(nz), "p0": tuple(np.asarray(p0, f32).tolist()), "p1": tuple(np.asarray(p1, f32).tolist()),
+                       "density": None if density is None else np.asarray(density, f32).reshape(-1)})
+        self.log.append(("MakeNamedMedium", name, kw))
+        if type not in ("homogeneous", "heterogeneous"):
+            raise B200Error(f'Medium "{type}" is outside the hot path (homogeneous, heterogeneous)')
         if preset:
             raise B200Error("named medium presets (get_medium_scattering_properties) are outside the hot path: give sigma_a / sigma_s")
         r = np.zeros(1, MEDIUM_DTYPE)[0]
         sa = np.full(3, sigma_a, f32) if np.isscalar(sigma_a) else np.asarray(sigma_a, f32)
         ss = np.full(3, sigma_s, f32) if np.isscalar(sigma_s) else np.asarray(sigma_s, f32)
         r["sigma_a"], r["sigma_s"], r["g"] = sa * f32(scale), ss * f32(scale), g
+        if type == "heterogeneous":
+            if density is None:
+                raise B200Error(f'No "density" values provided for heterogeneous medium "{name}"')
+            dens = np.asarray(density, f32).reshape(-1)
+            if len(dens) != int(nx) * int(ny) * int(nz):
+                raise B200Error(f'GridDensityMedium "{name}" has {len(dens)} density values; expected nx*ny*nz = {int(nx) * int(ny) * int(nz)}')
+            st = r["sigma_a"] + r["sigma_s"]
+            if not (st[0] == st[1] == st[2]):
+                warnings.warn(f'GridDensityMedium "{name}" requires a spectrally uniform sigma_t; using the first channel, {float(st[0])}')
+            pa, pb = np.asarray(p0, f32), np.asarray(p1, f32)
+            m2w = self.ctm * Transform.translate(pa) * Transform.scale(*(pb - pa))
+            self._grids.append(DensityGrid(dens, nx, ny, nz, m2w.m, m2w.m_inv))
+            r["grid"] = len(self._grids)
         self._media_index[name] = len(self._media)  # HashMap::insert replaces the entry; primitives created earlier keep the old Arc
         self._media.append(r)
 
@@ -961,6 +1010,7 @@ class SceneBuilder:
             fs.instances = inst
         if self._media:
             fs.media = np.array(self._media, MEDIUM_DTYPE)
+            fs.grids = list(self._grids)
             pm = np.concatenate(pmedia)
             if len(pm) and (pm >= 0).any():
                 fs.prim_media = np.ascontiguousarray(pm.view(MEDIUM_INTERFACE_DTYPE).reshape(-1))
@@ -1213,7 +1263,8 @@ class Scene:
         self.device = device
         h = C.c_void_p()
         d = flat.desc()
-        _check(self.lib.pbrt_b200_scene_create(C.byref(d), device, C.byref(h)), "pbrt_b200_scene_create")
+        grids = flat.grid_table()
+        _check(self.lib.pbrt_b200_scene_create_with_grids(C.byref(d), _ptr(grids), len(grids), device, C.byref(h)), "pbrt_b200_scene_create")
         self.handle = h
 
     def close(self):

@@ -55,6 +55,12 @@ def _params(kind, name, kw):
             out.append(f'"point {k}" [{_nums(v)}]')
         elif k == "scale" and kind == "MakeNamedMedium":
             out.append(f'"float scale" [{_num(v)}]')
+        elif kind == "MakeNamedMedium" and k in ("nx", "ny", "nz"):
+            out.append(f'"integer {k}" [{int(v)}]')
+        elif kind == "MakeNamedMedium" and k in ("p0", "p1"):
+            out.append(f'"point {k}" [{_nums(v)}]')
+        elif kind == "MakeNamedMedium" and k == "density":
+            out.append(f'"float density" [{_nums(v)}]')
         elif k in _RGB_KEYS or k in ("sigma_a", "sigma_s") or (k == "eta" and name == "metal"):
             out.append(f'"rgb {k}" [{_rgb(v)}]')
         elif k == "samples":

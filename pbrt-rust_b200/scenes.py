@@ -401,6 +401,103 @@ def fog_box_scene(xres=128, yres=128, spp=16, maxdepth=5, sampler="sobol", camer
     return SceneSetup("V1-fog-box", flat, make, "matte box in haze, smoke cube (material-less boundary), dye-filled glass sphere, mirror; volpath")
 
 
+def smoke_density(nx=14, ny=11, nz=9, seed=7):
+    """A seeded smoke field for GridDensityMedium, density[(z * ny + y) * nx + x]: fbm noise shaped into a blob, an empty (zero) border
+    of one voxel on every face and two empty spherical pockets inside."""
+    z, y, x = np.meshgrid(np.arange(nz), np.arange(ny), np.arange(nx), indexing="ij")
+    p = np.stack([(x + 0.5) / nx, (y + 0.5) / ny, (z + 0.5) / nz], -1).reshape(-1, 3).astype(f32)
+    r = np.linalg.norm((p - f32(0.5)) * np.array([1.0, 1.1, 1.3], f32), axis=1)
+    d = np.clip(f32(1.6) * (f32(0.55) - r) + f32(0.9) * fbm(p * f32(3.0), seed=seed, octaves=3), 0.0, None).astype(f32) * f32(4.0)
+    for c, rad in (((0.35, 0.45, 0.5), 0.16), ((0.65, 0.6, 0.4), 0.12)):
+        d[np.linalg.norm(p - np.array(c, f32), axis=1) < rad] = 0.0
+    d = d.reshape(nz, ny, nx)
+    d[0, :, :] = d[-1, :, :] = d[:, 0, :] = d[:, -1, :] = d[:, :, 0] = d[:, :, -1] = 0.0
+    return np.ascontiguousarray(d.reshape(-1), f32)
+
+
+def smoke_box_scene(xres=128, yres=128, spp=16, maxdepth=5, sampler="sobol", camera_in_smoke=False, instanced=False, textured=False, density=None,
+                    seed=7, smoke=True):
+    """Heterogeneous media for the volpath integrator: the room of fog_box_scene (matte walls, a thin homogeneous "haze", a mirror, one
+    quad area light, one point light) with a GridDensityMedium "smoke" (grid.rs) of 14 x 11 x 9 voxels from smoke_density(seed).  The
+    grid's box is rotated and scaled non-uniformly (CTM x Translate(p0) x Scale(p1 - p0), with p0 / p1 not the unit box), and its
+    material-less boundary mesh -- made under the same transformation -- reaches past the grid box on its -x side and cuts the box off
+    on its +x side.  `camera_in_smoke`: the camera sits inside the boundary, in the smoke (Camera.medium = smoke).  `instanced`: the
+    boundary is an ObjectInstance.  `textured`: the back wall is a checkerboard-textured matte.  `density`: replaces the field (same
+    14 x 11 x 9 layout), e.g. all zeros.  `smoke=False`: the same scene with vacuum inside the boundary instead of the grid medium."""
+    nx, ny, nz = 14, 11, 9
+    dens = smoke_density(nx, ny, nz, seed) if density is None else np.asarray(density, f32)
+    b = H.SceneBuilder()
+    b.make_named_medium("haze", sigma_a=(0.01, 0.012, 0.02), sigma_s=(0.12, 0.12, 0.14), g=0.1)
+    b.medium_interface("", "haze")
+
+    def wall(col, *pts, mat="matte", **kw):
+        b.material(mat, **({"Kd": col} if mat == "matte" else kw))
+        P, I = quad(*pts)
+        b.shape("trianglemesh", P=P, indices=I)
+
+    wall((0.7, 0.7, 0.7), (-2, -4, 0), (2, -4, 0), (2, 2, 0), (-2, 2, 0))        # floor: a transition into the haze
+    b.attribute_begin()
+    b.medium_interface("haze", "haze")
+    wall((0.7, 0.7, 0.7), (-2, -4, 2.5), (-2, 2, 2.5), (2, 2, 2.5), (2, -4, 2.5))  # ceiling
+    if textured:
+        from . import textures as T
+        b.material("matte", Kd=T.Tex.checkerboard(T.Mapping2D.planar((0.8, 0, 0), (0, 0, 0.8), 0.1, 0.2), np.array([0.8, 0.8, 0.8], f32),
+                                                  np.array([0.2, 0.3, 0.6], f32), "none"))
+        P, I = quad((-2, 2, 0), (2, 2, 0), (2, 2, 2.5), (-2, 2, 2.5))
+        b.shape("trianglemesh", P=P, indices=I)
+    else:
+        wall((0.7, 0.7, 0.7), (-2, 2, 0), (2, 2, 0), (2, 2, 2.5), (-2, 2, 2.5))      # back
+    wall((0.6, 0.1, 0.1), (-2, -4, 0), (-2, 2, 0), (-2, 2, 2.5), (-2, -4, 2.5))  # left
+    wall((0.1, 0.5, 0.15), (2, -4, 0), (2, -4, 2.5), (2, 2, 2.5), (2, 2, 0))     # right
+    wall((0.7, 0.7, 0.7), (-2, -4, 0), (-2, -4, 2.5), (2, -4, 2.5), (2, -4, 0))  # behind the camera
+    wall(None, (1.9, 1.2, 0.4), (1.2, 1.95, 0.4), (1.2, 1.95, 1.9), (1.9, 1.2, 1.9), mat="mirror", Kr=0.9)
+    b.attribute_end()
+    b.attribute_begin()
+    b.medium_interface("haze", "haze")
+    b.area_light_source("diffuse", L=(14, 13, 11))
+    b.material("matte", Kd=0.0)
+    P, I = quad((-0.5, -0.5, 2.49), (-0.5, 0.5, 2.49), (0.5, 0.5, 2.49), (0.5, -0.5, 2.49))
+    b.shape("trianglemesh", P=P, indices=I)
+    b.attribute_end()
+    b.light_source("point", **{"from": (1.4, -1.5, 1.4), "I": (3.0, 3.0, 3.5)})
+    b.attribute_begin()
+    b.translate(-0.8, -0.6, 0.15)
+    b.rotate(25.0, 0, 0, 1)
+    b.rotate(-10.0, 1, 0, 0)
+    b.scale(1.5, 1.3, 1.7)
+    if smoke:
+        b.make_named_medium("smoke", type="heterogeneous", sigma_a=(0.5, 0.25, 0.125), sigma_s=(2.0, 2.25, 2.375), g=0.5, scale=1.0,
+                            density=dens, nx=nx, ny=ny, nz=nz, p0=(-0.1, 0.0, 0.05), p1=(1.0, 1.0, 0.95))
+    ctm = b.ctm
+    b.medium_interface("smoke" if smoke else "", "haze")
+    b.material("none")
+    P, I = box_mesh((-0.3, -0.05, 0.0), (0.85, 1.08, 1.0))
+    if instanced:
+        b.object_begin("smokebox")
+        b.shape("trianglemesh", P=P, indices=I)
+        b.object_end()
+        b.object_instance("smokebox")
+    else:
+        b.shape("trianglemesh", P=P, indices=I)
+    b.attribute_end()
+    if camera_in_smoke:
+        eye = (ctm.m @ np.array([0.3, 0.15, 0.5, 1.0], f32))[:3]
+        cam_w2c = H.Transform.look_at(tuple(eye), (0.6, 1.9, 1.1), (0, 0, 1))
+        b.medium_interface("", "smoke" if smoke else "")
+    else:
+        cam_w2c = H.Transform.look_at((0.0, -3.4, 1.0), (0.0, 0.0, 0.9), (0, 0, 1))
+    cam_medium = b.camera_medium()
+    flat = b.world_end()
+
+    def make(spp_=spp, res=(xres, yres), maxdepth_=maxdepth, sampler_=sampler, strategy="uniform", filt="box", rrthreshold=1.0, pixelbounds=None):
+        film = H.Film(res[0], res[1], filt)
+        cam = H.PerspectiveCamera(film, cam_w2c.inverse(), fov=55.0)
+        return H.VolPathIntegrator(cam, film, H.Sampler(sampler_, spp_), maxdepth=maxdepth_, lightsamplestrategy=strategy, rrthreshold=rrthreshold,
+                                   camera_medium=cam_medium, pixelbounds=pixelbounds)
+
+    return SceneSetup("V2-smoke-box", flat, make, "grid-density smoke (rotated, non-uniformly scaled, clipped boundary) in a hazy room; volpath")
+
+
 def _test_image(w=96, h=64, channels=3):
     """A small deterministic image (NOT a power of two: MIPMap::new resamples it): stripes, a ramp and a few bright texels."""
     y, x = np.mgrid[0:h, 0:w]
