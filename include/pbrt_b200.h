@@ -270,7 +270,9 @@ enum { PBRT_B200_LIGHTS_UNIFORM = 0, PBRT_B200_LIGHTS_POWER = 1, PBRT_B200_LIGHT
  * (src/integrators/whitted.rs).  0 = path keeps descriptors written before the field existed valid.         */
 enum { PBRT_B200_INTEGRATOR_PATH = 0, PBRT_B200_INTEGRATOR_DIRECT_ONE = 1, PBRT_B200_INTEGRATOR_DIRECT_ALL = 2,
        PBRT_B200_INTEGRATOR_WHITTED = 3,
-       PBRT_B200_INTEGRATOR_VOLPATH = 4 /* `Integrator "volpath"` (src/integrators/volpath.rs:82-262) with homogeneous media */ };
+       PBRT_B200_INTEGRATOR_VOLPATH = 4 /* `Integrator "volpath"` (src/integrators/volpath.rs:82-262) with homogeneous media */,
+       PBRT_B200_INTEGRATOR_BDPT = 5    /* `Integrator "bdpt"` (src/integrators/bdpt.rs) on surfaces; rendered by pbrt_b200_render_splat
+                                         * only, since its light-tracing strategies add to a second film                        */ };
 
 /* = PathIntegrator (src/integrators/path.rs:32-40,228-249); max_depth and pixel_bounds mean the same for
  * DirectLightingIntegrator (directlighting.rs:27-39,122-157) and WhittedIntegrator (whitted.rs), which ignore
@@ -487,6 +489,18 @@ typedef struct pbrt_b200_render_stats {
 int pbrt_b200_render(pbrt_b200_scene *scene, const pbrt_b200_render_desc *desc,
                      float *rgbw_out, pbrt_b200_render_stats *stats);
 
+/* pbrt_b200_render for the PBRT_B200_INTEGRATOR_BDPT kind: BDPTIntegrator::render (pbrt-v3 integrators/bdpt.cpp), whose t = 1
+ * strategies (light subpaths connected to the camera) land on arbitrary pixels through Film::add_splat.  rgbw_out is as for
+ * pbrt_b200_render; splat_out[3 * width * height] over film.cropped_pixel_bounds receives the splatted RGB sums and follows the
+ * same rules (added to, PBRT_B200_RENDER_OVERWRITE and PBRT_B200_RENDER_KEEP_ON_DEVICE apply to both buffers, tile and sample
+ * windows sum).  Resolve with pbrt_b200_film_resolve_splat(splat_scale = 1 / samples_per_pixel).  Refused with
+ * PBRT_B200_ERR_UNSUPPORTED: scenes with participating media, the 02sequence sampler, and max_depth outside
+ * [0, PBRT_B200_BDPT_MAX_DEPTH] (each of the up to 2 * max_depth + 3 subpath vertices of a sample is kept in
+ * device memory).  Any other integrator kind is PBRT_B200_ERR_INVALID here.                                                    */
+#define PBRT_B200_BDPT_MAX_DEPTH 64
+int pbrt_b200_render_splat(pbrt_b200_scene *scene, const pbrt_b200_render_desc *desc,
+                           float *rgbw_out, float *splat_out, pbrt_b200_render_stats *stats);
+
 /* Device and pinned-host blocks released by pbrt_b200_scene_destroy are kept in a per-process pool and handed to the
  * next scene (the reference drops its Scene after every WorldEnd, src/core/api.rs:1750-1755; re-allocating ~6 GB of
  * path state per render would dominate short renders).  This returns every cached block to the driver.             */
@@ -502,6 +516,10 @@ int pbrt_b200_light_distribution_lookup(pbrt_b200_scene *scene, uint32_t strateg
 /* Film::write_image arithmetic (src/core/film.rs:217-264): RGB->XYZ->RGB,
  * divide by weight, clamp at 0, scale.  rgb_out[3*npixels].  Host buffers.      */
 int pbrt_b200_film_resolve(const float *rgbw, uint64_t npixels, float scale, float *rgb_out);
+
+/* Film::write_image(splat_scale) (pbrt-v3 film.cpp:148-185): the weighted RGB of pbrt_b200_film_resolve, clamped at 0, plus
+ * splat_scale times the splat film (through the same RGB->XYZ->RGB round trip), times scale.  rgb_out[3*npixels].             */
+int pbrt_b200_film_resolve_splat(const float *rgbw, const float *splat, uint64_t npixels, float splat_scale, float scale, float *rgb_out);
 
 #ifdef __cplusplus
 }

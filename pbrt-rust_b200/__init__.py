@@ -6,5 +6,5 @@ with `importlib.import_module("pbrt-rust_b200")` or through `__graft_entry__.pac
 from . import api, host, paramset, plymesh, pbrtparser, scenes, spectrum  # noqa: F401
 from .api import API, RenderJob  # noqa: F401
 from .pbrtparser import pbrt_parse, pbrt_parse_string  # noqa: F401
-from .host import (B200Error, DirectLightingIntegrator, WhittedIntegrator, VolPathIntegrator, Film, FlatScene, PathIntegrator, PerspectiveCamera, Sampler, Scene, SceneBuilder, Transform, bvh_build,  # noqa: F401
+from .host import (B200Error, BDPTIntegrator, DirectLightingIntegrator, WhittedIntegrator, VolPathIntegrator, Film, FlatScene, PathIntegrator, PerspectiveCamera, Sampler, Scene, SceneBuilder, Transform, bvh_build,  # noqa: F401
                    load_library, make_rays)

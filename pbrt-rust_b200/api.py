@@ -744,9 +744,9 @@ class API:
         camera = self._make_camera(film)
         sampler = self._make_sampler()
         name, p = self.ro["integrator"]
-        if name not in ("path", "directlighting", "whitted", "volpath"):
+        if name not in ("path", "directlighting", "whitted", "volpath", "bdpt"):
             if name in KNOWN_INTEGRATORS:
-                raise B200Error(f'Integrator "{name}" is outside the device path ("path", "volpath", "directlighting", "whitted")')
+                raise B200Error(f'Integrator "{name}" is outside the device path ("path", "volpath", "bdpt", "directlighting", "whitted")')
             raise B200Error(f'Integrator "{name}" unknown.')
         maxdepth = p.find_one_int("maxdepth", 5)  # path.rs:225-253, directlighting.rs:125, whitted.rs:111
         pb = p.find_int("pixelbounds")
@@ -767,6 +767,14 @@ class API:
             cam_medium = self.builder.camera_medium()
             integ = H.VolPathIntegrator(camera, film, sampler, maxdepth=maxdepth, rrthreshold=rr, lightsamplestrategy=strategy, pixelbounds=pixelbounds,
                                         camera_medium=cam_medium)
+        elif name == "bdpt":  # bdpt.rs / pbrt-v3 CreateBDPTIntegrator (bdpt.cpp:448-480)
+            if sampler.kind == H.SAMPLER_ZEROTWO:
+                raise B200Error('Integrator "bdpt" needs the sobol or halton sampler on the device path (as volpath does)')
+            vs, vw = p.find_one_bool("visualizestrategies", False), p.find_one_bool("visualizeweights", False)
+            if vs or vw:
+                raise B200Error('Integrator "bdpt": visualizestrategies / visualizeweights are not rendered on the device')
+            strategy = p.find_one_string("lightsamplestrategy", "power")
+            integ = H.BDPTIntegrator(camera, film, sampler, maxdepth=maxdepth, lightsamplestrategy=strategy, pixelbounds=pixelbounds)
         elif name == "directlighting":  # directlighting.rs:146-156
             st = p.find_one_string("strategy", "all")
             if st not in ("one", "all"):
@@ -795,7 +803,11 @@ class API:
         max_prims = ap.find_one_int("maxnodeprims", 4)
         ap.report_unused()
         flat = self.builder.world_end(max_prims=max_prims, split_method=split)
-        if self.have_scattering_media and name != "volpath":
+        if name == "bdpt":
+            self.builder._medium_names = self._medium_names()
+            if len(flat.media) or self.builder.camera_medium() >= 0:
+                raise B200Error('Integrator "bdpt" renders surfaces only: the scene has participating media (use "volpath")')
+        if self.have_scattering_media and name not in ("volpath", "bdpt"):
             warnings.warn(f'Scene has scattering media but "{name}" integrator doesn\'t support volume scattering.')
         return RenderJob(flat, integ, filename, (split, max_prims))
 

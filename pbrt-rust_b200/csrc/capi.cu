@@ -1021,3 +1021,19 @@ extern "C" int pbrt_b200_film_resolve(const float* rgbw, uint64_t npixels, float
     }
     return PBRT_B200_OK;
 }
+
+// Film::write_image(splat_scale) (pbrt-v3 film.cpp:148-185): the weighted RGB clamped at 0, plus splat_scale x the splat film
+extern "C" int pbrt_b200_film_resolve_splat(const float* rgbw, const float* splat, uint64_t npixels, float splat_scale, float scale, float* rgb_out) {
+    if (npixels && (!rgbw || !splat || !rgb_out)) return fail(PBRT_B200_ERR_INVALID, "film_resolve_splat: null argument");
+    int rc = pbrt_b200_film_resolve(rgbw, npixels, 1.0f, rgb_out);
+    if (rc) return rc;
+    for (uint64_t i = 0; i < npixels; ++i) {
+        const float* p = splat + 3 * i;
+        const float X = 0.412453f * p[0] + 0.357580f * p[1] + 0.180423f * p[2];
+        const float Y = 0.212671f * p[0] + 0.715160f * p[1] + 0.072169f * p[2];
+        const float Z = 0.019334f * p[0] + 0.119193f * p[1] + 0.950227f * p[2];
+        const float c[3] = {3.240479f * X - 1.537150f * Y - 0.498535f * Z, -0.969256f * X + 1.875991f * Y + 0.041556f * Z, 0.055648f * X - 0.204043f * Y + 1.057311f * Z};
+        for (int k = 0; k < 3; ++k) rgb_out[3 * i + k] = (rgb_out[3 * i + k] + splat_scale * c[k]) * scale;
+    }
+    return PBRT_B200_OK;
+}

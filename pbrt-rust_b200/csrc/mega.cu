@@ -7,26 +7,6 @@
 
 namespace pb {
 
-// FilmTile::add_sample without the warp aggregation of film_add_sample (the lanes of the one-kernel forms are not converged)
-PB_D void film_add_sample_lane(const RenderDev& R, float2 pfilm, rgb L) {
-    const float rx = R.filter_radius[0], ry = R.filter_radius[1];
-    const float ly = lum(L);
-    if (ly > R.max_sample_luminance) L = L * rgb(R.max_sample_luminance / ly);
-    const float dx = pfilm.x - 0.5f, dy = pfilm.y - 0.5f;
-    const int p0x = max((int)ceilf(dx - rx), R.crop[0]), p0y = max((int)ceilf(dy - ry), R.crop[1]);
-    const int p1x = min((int)floorf(dx + rx) + 1, R.crop[2]), p1y = min((int)floorf(dy + ry) + 1, R.crop[3]);
-    const int width = R.crop[2] - R.crop[0];
-    for (int y = p0y; y < p1y; ++y)
-        for (int x = p0x; x < p1x; ++x) {
-            float fx = fabsf(((float)x - dx) * R.inv_filter_radius[0] * 16.0f);
-            float fy = fabsf(((float)y - dy) * R.inv_filter_radius[1] * 16.0f);
-            int ix = min((int)floorf(fx), 15), iy = min((int)floorf(fy), 15);
-            float fw = __ldg(R.filter_table + iy * 16 + ix);
-            rgb c = L * rgb(1.0f) * rgb(fw);
-            atomicAdd(R.film + (size_t)(y - R.crop[1]) * width + (x - R.crop[0]), make_float4(c.r, c.g, c.b, fw));
-        }
-}
-
 // The (0,2)-sequence sampler under the PathIntegrator, one kernel: a tile's paths are inherently serial (every draw of
 // every path advances the tile's PCG32), so the wavefront form spends its time launching 13 kernels per path segment for a
 // few hundred threads.  Here ONE thread per tile (one warp per CTA, lane 0 working) walks its tile's pixels, samples and

@@ -615,6 +615,26 @@ PB_D void film_add_sample(const RenderDev& R, float2 pfilm, rgb L, bool active) 
         }
 }
 
+// FilmTile::add_sample without the warp aggregation of film_add_sample (the lanes of the one-kernel forms are not converged)
+PB_D void film_add_sample_lane(const RenderDev& R, float2 pfilm, rgb L) {
+    const float rx = R.filter_radius[0], ry = R.filter_radius[1];
+    const float ly = lum(L);
+    if (ly > R.max_sample_luminance) L = L * rgb(R.max_sample_luminance / ly);
+    const float dx = pfilm.x - 0.5f, dy = pfilm.y - 0.5f;
+    const int p0x = max((int)ceilf(dx - rx), R.crop[0]), p0y = max((int)ceilf(dy - ry), R.crop[1]);
+    const int p1x = min((int)floorf(dx + rx) + 1, R.crop[2]), p1y = min((int)floorf(dy + ry) + 1, R.crop[3]);
+    const int width = R.crop[2] - R.crop[0];
+    for (int y = p0y; y < p1y; ++y)
+        for (int x = p0x; x < p1x; ++x) {
+            float fx = fabsf(((float)x - dx) * R.inv_filter_radius[0] * 16.0f);
+            float fy = fabsf(((float)y - dy) * R.inv_filter_radius[1] * 16.0f);
+            int ix = min((int)floorf(fx), 15), iy = min((int)floorf(fy), 15);
+            float fw = __ldg(R.filter_table + iy * 16 + ix);
+            rgb c = L * rgb(1.0f) * rgb(fw);
+            atomicAdd(R.film + (size_t)(y - R.crop[1]) * width + (x - R.crop[0]), make_float4(c.r, c.g, c.b, fw));
+        }
+}
+
 // ---------------------------------------------------------------------------
 // K1: raygen
 // ---------------------------------------------------------------------------
@@ -1356,5 +1376,19 @@ void launch_zt_mega(const RenderDev& R, const RenderDev* rdev, uint32_t lanes, u
 void launch_vol_mega(const RenderDev& R, const RenderDev* rdev, unsigned long long total_items, int camera_medium, bool full, const DevGrid* grids, int grid,
                      cudaStream_t stream);
 int vol_mega_blocks_per_sm(bool full, bool grids);
+
+// ... and in bdpt.cu: PerspectiveCamera's importance functions need the inverse matrices, which the host computes once per call
+struct BdptCam {
+    float c2w[16], w2c[16], c2r[16];
+    f3 fwd;             // CameraToWorld(0, 0, 1) as a vector: cos(theta) of a ray leaving the lens
+    f3 n_lens;          // ... as a normal: the lens interaction's n
+    float A;            // image-plane area at z = 1 (pbrt-v3 perspective.cpp:55-62)
+    float lens_radius, focal_distance;
+    int sb[4];          // Film::get_sample_bounds
+    const float* spot_l2w;  // [n_lights][16] LightToWorld of spot lights (inverse of world_to_light), device memory
+};
+size_t bdpt_vertex_bytes();
+int bdpt_blocks_per_sm(bool inst);
+void launch_bdpt(const RenderDev& R, const BdptCam& C, void* verts, float* splat, unsigned long long total_items, bool inst, int grid, cudaStream_t stream);
 
 }  // namespace pb

@@ -962,8 +962,46 @@ extern "C" int pbrt_b200_light_distribution_lookup(pbrt_b200_scene* sc, uint32_t
     return PBRT_B200_OK;
 }
 
-extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc* rd, float* rgbw_out, pbrt_b200_render_stats* stats) {
-    if (!sc || !rd || !rgbw_out) return fail(PBRT_B200_ERR_INVALID, "render: null argument");
+// Matrix4x4::inverse (Gauss-Jordan with full pivoting, transform.rs:78-145), row-major; the BDPT camera and spot lights need inverses
+static void m4_inverse(const float* m, float* out) {
+    int indxc[4] = {0, 0, 0, 0}, indxr[4] = {0, 0, 0, 0}, ipiv[4] = {0, 0, 0, 0};
+    float a[4][4];
+    for (int i = 0; i < 16; ++i) a[i / 4][i % 4] = m[i];
+    for (int i = 0; i < 4; ++i) {
+        int irow = 0, icol = 0;
+        float big = 0.0f;
+        for (int j = 0; j < 4; ++j)
+            if (ipiv[j] != 1)
+                for (int k = 0; k < 4; ++k)
+                    if (ipiv[k] == 0 && std::fabs(a[j][k]) >= big) { big = std::fabs(a[j][k]); irow = j; icol = k; }
+        ipiv[icol] += 1;
+        if (irow != icol) for (int k = 0; k < 4; ++k) std::swap(a[irow][k], a[icol][k]);
+        indxr[i] = irow; indxc[i] = icol;
+        const float pivinv = 1.0f / a[icol][icol];
+        a[icol][icol] = 1.0f;
+        for (int j = 0; j < 4; ++j) a[icol][j] *= pivinv;
+        for (int j = 0; j < 4; ++j)
+            if (j != icol) {
+                const float save = a[j][icol];
+                a[j][icol] = 0.0f;
+                for (int k = 0; k < 4; ++k) a[j][k] -= a[icol][k] * save;
+            }
+    }
+    for (int i = 0; i < 4; ++i) {
+        const int j = 3 - i;
+        if (indxr[j] != indxc[j]) for (int k = 0; k < 4; ++k) std::swap(a[k][indxr[j]], a[k][indxc[j]]);
+    }
+    for (int i = 0; i < 16; ++i) out[i] = a[i / 4][i % 4];
+}
+static f3 m4_point_host(const float* M, f3 p) {  // Transform::transform_point (transform.rs:413-431)
+    const float xp = p.x * M[0] + p.y * M[1] + p.z * M[2] + M[3], yp = p.x * M[4] + p.y * M[5] + p.z * M[6] + M[7];
+    const float zp = p.x * M[8] + p.y * M[9] + p.z * M[10] + M[11], wp = p.x * M[12] + p.y * M[13] + p.z * M[14] + M[15];
+    if (wp == 1.0f) return f3(xp, yp, zp);
+    return f3(xp / wp, yp / wp, zp / wp);
+}
+
+// splat_out: the BDPT integrator's second film (pbrt_b200_render_splat); nullptr for pbrt_b200_render
+static int render_impl(pbrt_b200_scene* sc, const pbrt_b200_render_desc* rd, float* rgbw_out, float* splat_out, pbrt_b200_render_stats* stats) {
     if (rd->sampler.kind > PBRT_B200_SAMPLER_ZEROTWO) return fail(PBRT_B200_ERR_UNSUPPORTED, "render: sampler outside the hot path (sobol, halton, 02sequence)");
     if (rd->sampler.samples_per_pixel == 0) return fail(PBRT_B200_ERR_INVALID, "render: samples_per_pixel is 0");
     const bool zt = rd->sampler.kind == PBRT_B200_SAMPLER_ZEROTWO;
@@ -975,9 +1013,24 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
     }
     if (rd->integrator.light_sample_strategy > PBRT_B200_LIGHTS_SPATIAL) return fail(PBRT_B200_ERR_INVALID, "render: unknown light_sample_strategy");
     const uint32_t ikind = rd->integrator.kind;
-    if (ikind > PBRT_B200_INTEGRATOR_VOLPATH) return fail(PBRT_B200_ERR_INVALID, "render: unknown integrator kind");
+    if (ikind > PBRT_B200_INTEGRATOR_BDPT) return fail(PBRT_B200_ERR_INVALID, "render: unknown integrator kind");
+    const bool bd = ikind == PBRT_B200_INTEGRATOR_BDPT;
+    if (bd != (splat_out != nullptr))
+        return fail(PBRT_B200_ERR_INVALID, bd ? "render: the bdpt integrator renders through pbrt_b200_render_splat (its light-tracing strategies need a splat film)"
+                                              : "render_splat: only the bdpt integrator renders through pbrt_b200_render_splat");
+    if (bd) {
+        if (zt) return fail(PBRT_B200_ERR_UNSUPPORTED, "render: bdpt needs the sobol or halton sampler");
+        if (sc->dev.n_media || rd->integrator.camera_medium >= 0)
+            return fail(PBRT_B200_ERR_UNSUPPORTED, "render: bdpt renders surfaces only; scenes with participating media need volpath");
+        if (rd->integrator.max_depth < 0 || rd->integrator.max_depth > PBRT_B200_BDPT_MAX_DEPTH) {
+            char msg[160];
+            snprintf(msg, sizeof msg, "render: bdpt maxdepth %d outside [0, %d] (every subpath vertex of a sample is kept in device memory)",
+                     rd->integrator.max_depth, PBRT_B200_BDPT_MAX_DEPTH);
+            return fail(PBRT_B200_ERR_UNSUPPORTED, msg);
+        }
+    }
     const bool vol = ikind == PBRT_B200_INTEGRATOR_VOLPATH;
-    const bool path_like = ikind == PBRT_B200_INTEGRATOR_PATH || vol;  // no recursion state
+    const bool path_like = ikind == PBRT_B200_INTEGRATOR_PATH || vol || bd;  // no recursion state
     if (vol) {
         if (zt) return fail(PBRT_B200_ERR_UNSUPPORTED, "render: volpath needs the sobol or halton sampler");
         if (rd->integrator.camera_medium < -1 || rd->integrator.camera_medium >= (int64_t)sc->dev.n_media)
@@ -1055,8 +1108,16 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
         if (fit < 256) return fail(PBRT_B200_ERR_UNSUPPORTED, "render: too many lights for one whitted / directlighting \"all\" surface evaluation");
         if (capacity > fit) capacity = (uint32_t)(fit & ~255ull);
     }
-    // volpath: one slot per thread of the megakernel's single resident wave
+    // volpath / bdpt: one slot per thread of the megakernel's single resident wave
     int vol_grid = 0;
+    if (bd) {
+        int smc = 148;
+        cudaDeviceGetAttribute(&smc, cudaDevAttrMultiProcessorCount, sc->device);
+        const int per_sm = bdpt_blocks_per_sm(sc->dev.n_instances || sc->dev.n_sphere_lights || sc->dev.material_ext);
+        const unsigned long long want = (total_items + (unsigned long long)PB_VOL_BLOCK - 1ull) / (unsigned long long)PB_VOL_BLOCK;
+        vol_grid = (int)std::max<unsigned long long>(1ull, std::min<unsigned long long>((unsigned long long)smc * (unsigned long long)std::max(per_sm, 1), want));
+        capacity = ((uint32_t)vol_grid * (uint32_t)PB_VOL_BLOCK + 255u) & ~255u;
+    }
     if (vol) {
         int smc = 148, per_sm = 1;
         cudaDeviceGetAttribute(&smc, cudaDevAttrMultiProcessorCount, sc->device);
@@ -1067,7 +1128,7 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
     }
     if (capacity == 0) capacity = 256;
     if ((rc = ensure_buffers(st, &capacity))) return rc;
-    if (vol && capacity < (uint32_t)vol_grid * (uint32_t)PB_VOL_BLOCK) vol_grid = (int)(capacity / (uint32_t)PB_VOL_BLOCK);
+    if ((vol || bd) && capacity < (uint32_t)vol_grid * (uint32_t)PB_VOL_BLOCK) vol_grid = (int)(capacity / (uint32_t)PB_VOL_BLOCK);
     lap("buffers");
     RenderDev R = st->buffers->dev;
     R.capacity = capacity;
@@ -1212,9 +1273,9 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
     const bool timing = stats != nullptr && !zt;  // tile-serial mode runs ~10^5 tiny iterations: no per-phase events
     uint64_t launches = 0;
     // ---- Sobol' sample tables (sobol_tab_block) for the path integrator's global-sampler runs
-    bool sample_prepass = !zt && !R.rec.kind && !vol;  // k_sample_block serves every path the tables do not
+    bool sample_prepass = !zt && !R.rec.kind && !vol && !bd;  // k_sample_block serves every path the tables do not
     R.u8 = nullptr;
-    if (!zt && !R.rec.kind && !vol && S.kind == PBRT_B200_SAMPLER_SOBOL && S.log2_resolution > 0 && !getenv("PBRT_B200_NO_SOBOL_TABLES")) {
+    if (!zt && !R.rec.kind && !vol && !bd && S.kind == PBRT_B200_SAMPLER_SOBOL && S.log2_resolution > 0 && !getenv("PBRT_B200_NO_SOBOL_TABLES")) {
         const uint32_t sbw = (uint32_t)(sb[2] - sb[0]), sbh = (uint32_t)(sb[3] - sb[1]);
         // a path shading at bounce b < max_depth reads dimensions [s_dim, s_dim + 8) with s_dim <= 5 + 8b (camera 5, per bounce at most
         // light choice 1 + light 2 + scattering 2 + BSDF 2 + roulette 1): the tables serve every block iff they hold 5 + 8 * max_depth dimensions
@@ -1281,10 +1342,56 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
         PB_CUDA_TRY(cudaGetLastError());
         st->sp_eager_pending = false;
     }
-    if (vol && R.sp.enabled && R.sp.lazy)
-        return fail(PBRT_B200_ERR_UNSUPPORTED, "render: volpath with lightsamplestrategy \"spatial\" needs the eagerly built voxel table (voxels x lights <= 2^25)");
+    if ((vol || bd) && R.sp.enabled && R.sp.lazy)
+        return fail(PBRT_B200_ERR_UNSUPPORTED, "render: volpath / bdpt with lightsamplestrategy \"spatial\" needs the eagerly built voxel table (voxels x lights <= 2^25)");
+    // bdpt: the splat film (device pointer supplied, or a scratch film added back to the host buffer) and the subpath vertices
+    float* splat_dev = nullptr;
+    size_t splat_block = 0, verts_block = 0, spot_block = 0;
+    void* verts = nullptr;
+    float* spot_dev = nullptr;
+    if (bd) {
+        if (own_film) {
+            splat_dev = reinterpret_cast<float*>(pool_alloc(npix * 3 * sizeof(float), &splat_block));
+            if (!splat_dev) return fail(PBRT_B200_ERR_CUDA, "render: out of device memory for the splat film");
+            PB_CUDA_TRY(cudaMemsetAsync(splat_dev, 0, npix * 3 * sizeof(float), stream));
+        } else splat_dev = splat_out;
+        const size_t per_slot = (size_t)(2 * R.max_depth + 3) * bdpt_vertex_bytes();
+        verts = pool_alloc(std::max<size_t>((size_t)capacity * per_slot, 256), &verts_block);
+        if (!verts) { if (splat_block) pool_free(splat_dev, splat_block); return fail(PBRT_B200_ERR_CUDA, "render: out of device memory for the bdpt subpath vertices"); }
+    }
+    ZtRelease splat_release{splat_block ? splat_dev : nullptr, splat_block}, verts_release{verts, verts_block};
+    BdptCam bcam;
+    std::memset(&bcam, 0, sizeof bcam);
+    if (bd) {  // PerspectiveCamera::new's image-plane area and the inverses of camera and spot-light matrices (pbrt-v3 perspective.cpp:55-62)
+        const pbrt_b200_camera& cm = rd->camera;
+        std::memcpy(bcam.c2w, cm.camera_to_world, sizeof bcam.c2w);
+        m4_inverse(cm.camera_to_world, bcam.w2c);
+        m4_inverse(cm.raster_to_camera, bcam.c2r);
+        f3 pmin = m4_point_host(cm.raster_to_camera, f3(0.f, 0.f, 0.f));
+        f3 pmax = m4_point_host(cm.raster_to_camera, f3((float)rd->film.full_resolution[0], (float)rd->film.full_resolution[1], 0.f));
+        pmin = f3(pmin.x / pmin.z, pmin.y / pmin.z, pmin.z / pmin.z); pmax = f3(pmax.x / pmax.z, pmax.y / pmax.z, pmax.z / pmax.z);
+        bcam.A = std::fabs((pmax.x - pmin.x) * (pmax.y - pmin.y));
+        bcam.fwd = f3(cm.camera_to_world[2], cm.camera_to_world[6], cm.camera_to_world[10]);
+        bcam.n_lens = f3(bcam.w2c[8], bcam.w2c[9], bcam.w2c[10]);
+        bcam.lens_radius = cm.lens_radius; bcam.focal_distance = cm.focal_distance;
+        for (int i = 0; i < 4; ++i) bcam.sb[i] = sb[i];
+        std::vector<float> l2w(16 * std::max<size_t>(st->lights_host.size(), 1), 0.0f);
+        for (size_t i = 0; i < st->lights_host.size(); ++i)
+            if (st->lights_host[i].type == PBRT_B200_LIGHT_SPOT) m4_inverse(st->lights_host[i].world_to_light, l2w.data() + 16 * i);
+        spot_dev = reinterpret_cast<float*>(pool_alloc(l2w.size() * sizeof(float), &spot_block));
+        if (!spot_dev) return fail(PBRT_B200_ERR_CUDA, "render: out of device memory");
+        PB_CUDA_TRY(cudaMemcpyAsync(spot_dev, l2w.data(), l2w.size() * sizeof(float), cudaMemcpyHostToDevice, stream));
+        bcam.spot_l2w = spot_dev;
+    }
+    ZtRelease spot_release{spot_dev, spot_block};
     PB_CUDA_TRY(cudaEventRecord(ev0, stream));
-    if (vol) {
+    if (bd) {
+        if (total_items > 0) {
+            launch_bdpt(R, bcam, verts, splat_dev, total_items, sc->dev.n_instances || sc->dev.n_sphere_lights || sc->dev.material_ext, vol_grid, stream);
+            launches += 1;
+            PB_CUDA_TRY(cudaGetLastError());
+        }
+    } else if (vol) {
         if (total_items > 0) {
             // R in device memory for the out-of-line shade calls (as k_zt_mega)
             size_t rdev_bytes = 0;
@@ -1437,6 +1544,12 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
         }
         stats->iterations = c.iterations;
     }
+    if (bd && own_film) {  // the splat film: same rules as the rgbw film
+        std::vector<float> hs(npix * 3);
+        PB_CUDA_TRY(cudaMemcpy(hs.data(), splat_dev, hs.size() * sizeof(float), cudaMemcpyDeviceToHost));
+        if (rd->flags & PBRT_B200_RENDER_OVERWRITE) std::memcpy(splat_out, hs.data(), hs.size() * sizeof(float));
+        else for (size_t i = 0; i < hs.size(); ++i) splat_out[i] += hs[i];
+    }
     if (own_film) {
         // film tile merge (merge_film_tile, film.rs:142-161): device film -> pinned staging in chunks, each chunk added into
         // the caller's buffer while the next one is in flight
@@ -1479,4 +1592,13 @@ extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc
         lap("film d2h + merge");
     }
     return PBRT_B200_OK;
+}
+
+extern "C" int pbrt_b200_render(pbrt_b200_scene* sc, const pbrt_b200_render_desc* rd, float* rgbw_out, pbrt_b200_render_stats* stats) {
+    if (!sc || !rd || !rgbw_out) return fail(PBRT_B200_ERR_INVALID, "render: null argument");
+    return render_impl(sc, rd, rgbw_out, nullptr, stats);
+}
+extern "C" int pbrt_b200_render_splat(pbrt_b200_scene* sc, const pbrt_b200_render_desc* rd, float* rgbw_out, float* splat_out, pbrt_b200_render_stats* stats) {
+    if (!sc || !rd || !rgbw_out || !splat_out) return fail(PBRT_B200_ERR_INVALID, "render_splat: null argument");
+    return render_impl(sc, rd, rgbw_out, splat_out, stats);
 }

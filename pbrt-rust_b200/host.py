@@ -64,7 +64,8 @@ MAT_MATTE, MAT_PLASTIC, MAT_MIRROR, MAT_GLASS, MAT_METAL, MAT_UBER, MAT_SUBSTRAT
 LIGHT_POINT, LIGHT_DISTANT, LIGHT_SPOT, LIGHT_DIFFUSE, LIGHT_INFINITE = range(5)
 SAMPLER_SOBOL, SAMPLER_HALTON, SAMPLER_ZEROTWO = range(3)
 LIGHTS_UNIFORM, LIGHTS_POWER, LIGHTS_SPATIAL = range(3)
-INTEGRATOR_PATH, INTEGRATOR_DIRECT_ONE, INTEGRATOR_DIRECT_ALL, INTEGRATOR_WHITTED, INTEGRATOR_VOLPATH = range(5)
+INTEGRATOR_PATH, INTEGRATOR_DIRECT_ONE, INTEGRATOR_DIRECT_ALL, INTEGRATOR_WHITTED, INTEGRATOR_VOLPATH, INTEGRATOR_BDPT = range(6)
+BDPT_MAX_DEPTH = 64  # PBRT_B200_BDPT_MAX_DEPTH: the bdpt integrator keeps every subpath vertex of a sample in device memory
 SPLIT = {"sah": 0, "middle": 2, "equal": 3}
 
 
@@ -125,7 +126,7 @@ EXPORTS = ["pbrt_b200_last_error", "pbrt_b200_abi_version", "pbrt_b200_device_co
            "pbrt_b200_scene_destroy", "pbrt_b200_scene_world_bound", "pbrt_b200_intersect", "pbrt_b200_intersect_p", "pbrt_b200_intersect_dev",
            "pbrt_b200_intersect_p_dev", "pbrt_b200_render", "pbrt_b200_film_resolve", "pbrt_b200_light_distribution_lookup", "pbrt_b200_release_cached_memory", "pbrt_b200_tile_positions",
            "pbrt_b200_work_counter_open", "pbrt_b200_work_counter_fetch_add", "pbrt_b200_work_counter_fetch_max", "pbrt_b200_work_counter_load", "pbrt_b200_work_counter_store",
-           "pbrt_b200_work_counter_close"]
+           "pbrt_b200_work_counter_close", "pbrt_b200_render_splat", "pbrt_b200_film_resolve_splat"]
 
 
 class B200Error(RuntimeError):
@@ -158,6 +159,8 @@ def load_library():
     lib.pbrt_b200_intersect_p_dev.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
     lib.pbrt_b200_render.argtypes = [C.c_void_p, C.POINTER(RenderDesc), C.c_void_p, C.POINTER(RenderStats)]
     lib.pbrt_b200_film_resolve.argtypes = [C.c_void_p, C.c_uint64, C.c_float, C.c_void_p]
+    lib.pbrt_b200_render_splat.argtypes = [C.c_void_p, C.POINTER(RenderDesc), C.c_void_p, C.c_void_p, C.POINTER(RenderStats)]
+    lib.pbrt_b200_film_resolve_splat.argtypes = [C.c_void_p, C.c_void_p, C.c_uint64, C.c_float, C.c_float, C.c_void_p]
     lib.pbrt_b200_release_cached_memory.restype = None
     lib.pbrt_b200_light_distribution_lookup.argtypes = [C.c_void_p, C.c_uint32, C.c_uint32, C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p]
     lib.pbrt_b200_tile_positions.argtypes = [C.c_int, C.c_int, C.c_uint32]
@@ -1245,6 +1248,30 @@ class VolPathIntegrator(PathIntegrator):
         self.camera_medium = int(camera_medium)
 
 
+class BDPTIntegrator(PathIntegrator):
+    """BDPTIntegrator + create_bdpt_integrator (src/integrators/bdpt.rs; pbrt-v3 integrators/bdpt.cpp:448-480): maxdepth, the light
+    sample strategy (default "power"; "spatial" is looked up at the camera vertex) and pixelbounds.  Its light-tracing strategies splat
+    onto a second film, so it renders through Scene.render_splat; render() resolves both films with splat_scale = 1 / spp."""
+    name = "bdpt"
+    kind = INTEGRATOR_BDPT
+
+    def __init__(self, camera, film, sampler, maxdepth=5, lightsamplestrategy="power", pixelbounds=None, visualizestrategies=False,
+                 visualizeweights=False):
+        if visualizestrategies or visualizeweights:
+            raise B200Error('Integrator "bdpt": visualizestrategies / visualizeweights are not rendered on the device')
+        if int(maxdepth) < 0 or int(maxdepth) > BDPT_MAX_DEPTH:
+            raise B200Error(f'Integrator "bdpt": maxdepth {int(maxdepth)} is outside [0, {BDPT_MAX_DEPTH}] (every subpath vertex is kept in device memory)')
+        if lightsamplestrategy not in self.STRATEGY:
+            raise B200Error(f'Integrator "bdpt": unknown lightsamplestrategy "{lightsamplestrategy}" (uniform, power, spatial)')
+        super().__init__(camera, film, sampler, maxdepth=maxdepth, rrthreshold=1.0, lightsamplestrategy=lightsamplestrategy, pixelbounds=pixelbounds)
+
+    def render(self, scene, **kw):
+        """-> linear RGB image [h, w, 3] (Film::write_image(1 / spp)), stats."""
+        rgbw, splat, stats = scene.render_splat(self, **kw)
+        img = scene.film_resolve_splat(rgbw, splat, 1.0 / self.sampler.spp, self.film.scale)
+        return img.reshape(self.film.height, self.film.width, 3), stats
+
+
 class WhittedIntegrator(PathIntegrator):
     """WhittedIntegrator + create_whitted_integrator (src/integrators/whitted.rs:25-50,108-131)."""
     name = "whitted"
@@ -1327,6 +1354,33 @@ class Scene:
         rgbw = np.ascontiguousarray(rgbw, f32).reshape(-1, 4)
         out = np.zeros((len(rgbw), 3), f32)
         _check(self.lib.pbrt_b200_film_resolve(_ptr(rgbw), len(rgbw), scale, _ptr(out)), "pbrt_b200_film_resolve")
+        return out
+
+    def render_splat(self, integrator, rgbw=None, splat=None, tile_range=None, sample_range=None, device_ptrs=None, tile_interleave=None, flags=0,
+                     tile_order=0):
+        """pbrt_b200_render_splat -> ({r,g,b,w} sums [npix, 4], splat RGB sums [npix, 3], stats).  Buffers passed in are added to;
+        device_ptrs = (rgbw, splat) device pointers keeps both films on the device."""
+        film = integrator.film
+        stats = RenderStats()
+        if device_ptrs is not None:
+            d = integrator.desc(tile_range, sample_range, 0, RENDER_KEEP_ON_DEVICE | flags, tile_interleave, tile_order)
+            _check(self.lib.pbrt_b200_render_splat(self.handle, C.byref(d), device_ptrs[0], device_ptrs[1], C.byref(stats)), "pbrt_b200_render_splat")
+            return None, None, stats
+        if rgbw is None and splat is None:  # fresh films: the library overwrites them
+            rgbw = np.empty((film.height * film.width, 4), f32)
+            splat = np.empty((film.height * film.width, 3), f32)
+            flags |= RENDER_OVERWRITE
+        elif rgbw is None or splat is None:
+            raise B200Error("render_splat: pass both films or neither")
+        d = integrator.desc(tile_range, sample_range, 0, flags, tile_interleave, tile_order)
+        _check(self.lib.pbrt_b200_render_splat(self.handle, C.byref(d), _ptr(rgbw), _ptr(splat), C.byref(stats)), "pbrt_b200_render_splat")
+        return rgbw, splat, stats
+
+    def film_resolve_splat(self, rgbw, splat, splat_scale, scale=1.0):
+        rgbw = np.ascontiguousarray(rgbw, f32).reshape(-1, 4)
+        splat = np.ascontiguousarray(splat, f32).reshape(-1, 3)
+        out = np.zeros((len(rgbw), 3), f32)
+        _check(self.lib.pbrt_b200_film_resolve_splat(_ptr(rgbw), _ptr(splat), len(rgbw), splat_scale, scale, _ptr(out)), "pbrt_b200_film_resolve_splat")
         return out
 
 

@@ -243,6 +243,73 @@ def cornell_scene(xres=1024, yres=1024, spp=256, maxdepth=8, sampler="sobol"):
     return SceneSetup("S2-cornell", flat, make, "Cornell box, quad area light (2 triangle lights), matte + plastic, power light sampling")
 
 
+def caustic_scene(xres=256, yres=256, spp=64, maxdepth=8, sampler="sobol"):
+    """A caustic under a small light: a glass sphere on a matte floor in front of a matte back wall, lit by a small quad area
+    light above and behind it.  Most of the light that reaches the floor under the sphere went through the glass, the case in which
+    the path integrator converges slowly and the bdpt integrator's light subpaths help."""
+    b = H.SceneBuilder()
+    cam_w2c = H.Transform.look_at((0, 2.2, 5.5), (0, 0.4, 0), (0, 1, 0))
+    b.material("matte", Kd=(0.7, 0.7, 0.7))
+    P, I = quad((-4, 0, -4), (4, 0, -4), (4, 0, 4), (-4, 0, 4))
+    b.shape("trianglemesh", P=P, indices=I)
+    P, I = quad((-4, 0, -2), (-4, 4, -2), (4, 4, -2), (4, 0, -2))
+    b.shape("trianglemesh", P=P, indices=I)
+    b.attribute_begin()
+    b.area_light_source("diffuse", L=(120, 110, 95))
+    b.material("matte", Kd=0.0)
+    P, I = quad((-0.2, 3.0, -0.6), (-0.2, 3.0, -0.2), (0.2, 3.0, -0.2), (0.2, 3.0, -0.6))
+    b.shape("trianglemesh", P=P, indices=I)
+    b.attribute_end()
+    b.attribute_begin()
+    b.translate(0, 0.8, 0)
+    b.material("glass")
+    b.shape("sphere", radius=0.8)
+    b.attribute_end()
+    flat = b.world_end()
+
+    def make(spp_=spp, res=(xres, yres), maxdepth_=maxdepth, sampler_=sampler, strategy="power", filt="box", crop=(0.0, 1.0, 0.0, 1.0)):
+        film = H.Film(res[0], res[1], filt, crop=crop)
+        cam = H.PerspectiveCamera(film, cam_w2c.inverse(), fov=40.0)
+        return H.PathIntegrator(cam, film, H.Sampler(sampler_, spp_), maxdepth=maxdepth_, lightsamplestrategy=strategy)
+
+    return SceneSetup("caustic", flat, make, "glass sphere on a matte floor under a small quad area light (caustic)")
+
+
+def one_light_scene(light="spot", xres=48, yres=48, spp=16, maxdepth=4, sampler="sobol"):
+    """A matte floor and back wall with a plastic box, lit by ONE light of kind `light`: "spot", "point", "sphere" (a two-sided sphere
+    area light) or "sphere_one_sided" (one-sided: the reference's cone sample leaves the sampled normal at zero, so it emits through
+    BSDF-sampled rays and light subpaths but not through light sampling).  For checking each light's sampling functions alone."""
+    b = H.SceneBuilder()
+    cam_w2c = H.Transform.look_at((0, 1.6, 5.0), (0, 0.6, 0), (0, 1, 0))
+    b.material("matte", Kd=(0.6, 0.6, 0.6))
+    P, I = quad((-4, 0, -4), (4, 0, -4), (4, 0, 4), (-4, 0, 4))
+    b.shape("trianglemesh", P=P, indices=I)
+    P, I = quad((-4, 0, -1.5), (-4, 4, -1.5), (4, 4, -1.5), (4, 0, -1.5))
+    b.shape("trianglemesh", P=P, indices=I)
+    b.material("plastic", Kd=(0.2, 0.4, 0.7), Ks=0.3, roughness=0.1)
+    P, I = box_mesh((-0.9, 0.0, -0.6), (-0.1, 0.8, 0.2))
+    b.shape("trianglemesh", P=P, indices=I)
+    if light == "spot":
+        b.light_source("spot", **{"from": (0.5, 2.8, 1.5), "to": (0.0, 0.0, -0.5), "coneangle": 35.0, "conedelta": 10.0, "I": (12, 11, 10)})
+    elif light == "point":
+        b.light_source("point", **{"from": (0.5, 2.5, 1.0), "I": (8, 8, 8)})
+    else:
+        b.attribute_begin()
+        b.translate(0.8, 2.2, 0.6)
+        b.area_light_source("diffuse", L=(6, 6, 5.5), twosided=(light == "sphere"))
+        b.material("matte", Kd=0.0)
+        b.shape("sphere", radius=0.3)
+        b.attribute_end()
+    flat = b.world_end()
+
+    def make(spp_=spp, res=(xres, yres), maxdepth_=maxdepth, sampler_=sampler, strategy="power", filt="box"):
+        film = H.Film(res[0], res[1], filt)
+        cam = H.PerspectiveCamera(film, cam_w2c.inverse(), fov=45.0)
+        return H.PathIntegrator(cam, film, H.Sampler(sampler_, spp_), maxdepth=maxdepth_, lightsamplestrategy=strategy)
+
+    return SceneSetup(f"one-light-{light}", flat, make, f"floor, wall and box under one {light} light")
+
+
 def displaced_sphere_scene(nlong=1024, nlat=512, xres=1920, yres=1080, spp=512, maxdepth=5, sampler="sobol"):
     """S3 / config C3: nlong*nlat*2 triangles (1 048 576 at the defaults) on a displaced sphere with
     per-vertex normals, half plastic / half copper metal by octant parity, ground quad, one quad
